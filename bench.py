@@ -3,6 +3,11 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference|reference-gpu]
                     [--precision bf16|fp32] [--variant D|Y] [--batch B] [--track SECONDS] [--model mss|bs]
+                    [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step returned as DIR/<name>.npy (float32): the separated sources of the
+forward and --track runs, the complex estimate of --model bs as `est` (real and imaginary parts in a last axis of 2).
+Weights and inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
 Workload (BASELINE.json configs[1], "Variant D" of SURVEY.md F4): n_fft 2048, hop 1024, 6 layers,
 emb_dim 128, 4 heads, macaron ConvSwiGLU [384, 384], 4 sources; one step = one batch of 6-s 44.1 kHz
@@ -107,6 +112,27 @@ def make_state_dict(cfg, seed=0):
             if p.ndim == 1 and not n.endswith("rope.freqs"):
                 p.add_(0.1 * torch.randn(p.shape, generator=g))
     return model
+
+
+DUMP_BYTES = 64_000_000      # all files of one dump, .npy headers included
+NPY_HEADER = 128             # bytes of a .npy v1 header for the shapes dumped here
+
+
+def dump_outputs(out, directory, budget=DUMP_BYTES):
+    """Write each tensor of `out` (name -> tensor) as directory/<name>.npy in float32.  When the files would exceed
+    `budget` bytes together, every tensor is cut to the same fixed, seeded sample of its flattened elements (indices
+    in ascending order), so that dumps of two builds at the same arguments still compare element for element."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    total = sum(v.numel() for v in out.values())
+    keep = min(1.0, (budget - NPY_HEADER * len(out)) / (4 * total))
+    for name, v in out.items():
+        a = v.detach().to("cpu", torch.float32)
+        if keep < 1.0:
+            g = torch.Generator().manual_seed(0)
+            idx = torch.randperm(a.numel(), generator=g)[: int(a.numel() * keep)].sort().values
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(directory, name + ".npy"), a.numpy())
 
 
 class ClockSampler:
@@ -286,10 +312,12 @@ def run_bs(args, dev):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(args.steps):
-            model(spec)
+            est = model(spec)
         e1.record()
         torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / args.steps
+    if args.dump_outputs:
+        dump_outputs({"est": torch.view_as_real(est)}, args.dump_outputs)
     print(json.dumps({
         "metric": METRIC, "value": B * SEG / SR / (ms / 1e3), "unit": "audio-s/s", "n_gpus": 1, "steps": args.steps,
         "warmup": max(3, args.warmup), "ms_per_step": ms, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -463,7 +491,13 @@ def main():
                     help="BASELINE config 5: time data-parallel TRAINING steps of this configuration instead of inference")
     ap.add_argument("--train-seconds", type=float, default=0.0, help="seconds of audio per training sample (0 = the configuration's own)")
     ap.add_argument("--train-batch", type=int, default=1, help="training samples per GPU per step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed separation step returned (rank 0) as DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.train):
+        ap.error("--dump-outputs applies to the separation benchmarks of --impl b200 (not --train)")
     args.warmup = max(args.warmup, 3) if (args.impl == "b200" and args.train is None) else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -516,17 +550,18 @@ def main():
             dist.destroy_process_group()
 
     def timed(fn, steps):
+        """-> (ms over `steps` calls of fn, what the last call returned)."""
         sync_all()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         sync_all()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item())
+        return float(ms.item()), out
 
     def step_resident():
         with torch.no_grad():
@@ -574,8 +609,10 @@ def main():
 
         for _ in range(max(1, args.warmup // 3)):
             step_track()
-        ms = timed(step_track, args.steps)
+        ms, out = timed(step_track, args.steps)
         finish_group()
+        if rank == 0 and args.dump_outputs:
+            dump_outputs(out, args.dump_outputs)
         if rank == 0:
             print(json.dumps({
                 "metric": METRIC, "value": args.track * args.steps / (ms / 1e3), "unit": "audio-s/s", "n_gpus": world,
@@ -591,8 +628,10 @@ def main():
         step_resident()
     n0 = lib.tfl_launch_count()
     with ClockSampler(local) as clocks:
-        ms = timed(step_resident, args.steps)
+        ms, last = timed(step_resident, args.steps)
     launches = lib.tfl_launch_count() - n0
+    # host copy before the end-to-end steps run the model again; nothing of it is timed
+    last = {k: v.cpu() for k, v in last.items()} if args.dump_outputs else None
     for _ in range(2):
         step_e2e()
     drain_e2e()
@@ -615,6 +654,8 @@ def main():
     finish_group()          # ---- no collective below this line ----
     if rank != 0:
         return
+    if last is not None:
+        dump_outputs(last, args.dump_outputs)
 
     audio_s = world * B * SEG / SR
     value = audio_s * args.steps / (ms / 1e3)

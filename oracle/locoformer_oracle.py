@@ -221,7 +221,9 @@ def blocks_forward(x, sd, cfg, prefix="blocks"):
 # Whole models
 # --------------------------------------------------------------------------------------
 def _cast(sd, dtype):
-    return {k: v.detach().to(dtype) if v.is_floating_point() else v for k, v in sd.items()}
+    """Weights in the compute dtype; a weight that requires grad keeps its autograd graph (the training tests
+    differentiate the oracle forward with respect to the state_dict)."""
+    return {k: v.to(dtype) if v.is_floating_point() else v for k, v in sd.items()}
 
 
 def separator_forward(sd, cfg: dict, spec: torch.Tensor, dtype=torch.float32) -> torch.Tensor:

@@ -126,6 +126,41 @@ def test_bench_reference_arm_line(monkeypatch, capsys):
     assert line["e2e"] == {"value": line["value"], "unit": "audio-s/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
 
 
+def test_bench_dump_outputs_full_and_sampled(tmp_path):
+    """bench.py --dump-outputs: float32 .npy per source, whole when the arrays fit the budget, else the same seeded
+    sample of every array (identical from call to call) within it."""
+    import bench
+    g = torch.Generator().manual_seed(3)
+    out = {"vocals": torch.randn(2, 1000, generator=g, dtype=torch.float64), "drums": torch.randn(2, 1000, generator=g)}
+    bench.dump_outputs(out, str(tmp_path / "full"))
+    for k, v in out.items():
+        a = np.load(tmp_path / "full" / f"{k}.npy")
+        assert a.dtype == np.float32 and a.shape == (2, 1000)
+        assert np.array_equal(a, v.float().numpy())
+    budget = 4 * 1000 + 2 * bench.NPY_HEADER              # files of a quarter of the 4000 elements
+    for run in ("a", "b"):
+        bench.dump_outputs(out, str(tmp_path / run), budget=budget)
+    sizes = 0
+    for k, v in out.items():
+        a, b = np.load(tmp_path / "a" / f"{k}.npy"), np.load(tmp_path / "b" / f"{k}.npy")
+        assert a.dtype == np.float32 and a.shape == (500,) and np.array_equal(a, b)
+        assert np.isin(a, v.float().numpy().reshape(-1)).all()
+        sizes += os.path.getsize(tmp_path / "a" / f"{k}.npy")
+    assert sizes <= budget
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--dump-outputs", "d", "--train", "D"],
+                                  ["--dump-outputs", "d", "--impl", "reference"],
+                                  ["--dump-outputs", "d", "--impl", "reference-gpu"]])
+def test_bench_rejects_arguments_it_cannot_honour(monkeypatch, argv):
+    """No timed step, or a dump requested from a path that does not write one: an argument error before any work."""
+    import bench
+    monkeypatch.setattr("sys.argv", ["bench.py"] + argv)
+    with pytest.raises(SystemExit) as e:
+        bench.main()
+    assert e.value.code == 2
+
+
 def test_bench_train_dtype_names_the_operand_type():
     import bench
     assert bench.train_dtype(bench.TRAIN_CFGS["D"][0]) == "bf16"          # tcgen05 forward + bf16 mma.sync backward
