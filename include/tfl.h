@@ -79,6 +79,11 @@ int tfl_stft(const tfl_plan* plan, const void* packed, const float* audio, int b
 /* :141-146, :218-219.  spec [B, Tf, F, Cin] -> x [B, Tf, F, C] (conv 3x3 + gLN). */
 int tfl_enc_conv_gln(const tfl_plan* plan, const void* packed, const float* spec, int batch, int n_frames,
                      int n_freq, float* x, void* workspace, size_t ws_bytes, tfl_stream_t stream);
+/* The same stage in the arithmetic of `precision`: TFL_PRECISION_FP32 = tfl_enc_conv_gln; TFL_PRECISION_BF16 = the tf32
+ * mma.sync encoder that tfl_forward / tfl_separator_forward run in bf16 mode (spectrogram and weights rounded to tf32,
+ * fp32 sums, gLN statistics in double). */
+int tfl_enc_conv_gln_mode(const tfl_plan* plan, const void* packed, const float* spec, int batch, int n_frames,
+                          int n_freq, float* x, void* workspace, size_t ws_bytes, int precision, tfl_stream_t stream);
 /* :682-706.  x [rows, C] -> y [rows, C] with the gamma of (layer, axis, which) where
  * which = 0: ffn_norm.0, 1: ffn_norm.1, 2: attn_norm. */
 int tfl_rms_group_norm(const tfl_plan* plan, const void* packed, int layer, int axis, int which,

@@ -36,6 +36,7 @@ SIGNATURES = {  # name -> (restype, argtypes); must list every symbol of include
     "tfl_workspace_bytes": (_Z, [_P, _I, _I, _I, _I]),
     "tfl_stft": (_I, [_P, _P, _P, _I, _I, _P, _P]),
     "tfl_enc_conv_gln": (_I, [_P, _P, _P, _I, _I, _I, _P, _P, _Z, _P]),
+    "tfl_enc_conv_gln_mode": (_I, [_P, _P, _P, _I, _I, _I, _P, _P, _Z, _I, _P]),
     "tfl_rms_group_norm": (_I, [_P, _P, _I, _I, _I, _P, _P, _L, _P]),
     "tfl_conv_swiglu_ffn": (_I, [_P, _P, _I, _I, _I, _P, _I, _I, _I, _P, _Z, _I, _P]),
     "tfl_conv_swiglu_ffn_out": (_I, [_P, _P, _I, _I, _I, _P, _P, _I, _I, _I, _P, _Z, _I, _P]),

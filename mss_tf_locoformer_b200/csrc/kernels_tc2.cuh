@@ -65,8 +65,12 @@ static_assert(FFN2_REGS_CTRL + FFN2_REGS_PROD + 2 * FFN2_REGS_SWIGLU + FFN2_REGS
 #define FFN2_SETMAXNREG(dir, n) asm volatile("setmaxnreg." dir ".sync.aligned.u32 %0;" ::"n"(n))
 #endif
 
+// The A-tile producers hold one (row, group) item of at most 32 channels in registers (eight float4): wider norm
+// groups (emb_dim / num_groups > 32) run on ffn_tc_kernel, whose producers also have a loop over the group.
 inline bool ffn2_geometry(int C, int H, int KT, int G, Ffn2Geom* g) {
-  if (C % 32 != 0 || C > 128 || H % TC_HC != 0 || (C / G) % 4 != 0 || KT < 1 || KT > 8) return false;
+  if (C % 32 != 0 || C > 128 || H % TC_HC != 0 || G < 1 || C % G != 0 || (C / G) % 4 != 0 || C / G > 32 || KT < 1 ||
+      KT > 8)
+    return false;
   g->C = C; g->H = H; g->KT = KT; g->G = G;
   g->AR = 128 + KT - 1; g->TS = 128 - (KT - 1);
   g->NC = H / TC_HC;
@@ -99,9 +103,9 @@ inline bool ffn2_geometry(int C, int H, int KT, int G, Ffn2Geom* g) {
   return true;
 }
 
-inline size_t tc_ffn2_image_bytes(int C, int H, int K) {
+inline size_t tc_ffn2_image_bytes(int C, int H, int K, int G) {
   Ffn2Geom g;
-  if (!ffn2_geometry(C, H, K, 1, &g)) return 0;
+  if (!ffn2_geometry(C, H, K, G, &g)) return 0;
   return (size_t)g.NC * (K * g.KH + g.KS) * 2 * g.half_bytes;
 }
 
@@ -140,9 +144,9 @@ __global__ void tc_pack_ffn2_kernel(const float* __restrict__ w1, const float* _
   }
 }
 
-inline int tc_pack_ffn2(const float* w1, const float* w2, char* img, int C, int H, int K, cudaStream_t st) {
+inline int tc_pack_ffn2(const float* w1, const float* w2, char* img, int C, int H, int K, int G, cudaStream_t st) {
   Ffn2Geom g;
-  if (!ffn2_geometry(C, H, K, 1, &g)) return 0;
+  if (!ffn2_geometry(C, H, K, G, &g)) return 0;
   tc_pack_ffn2_kernel<<<592, 256, 0, st>>>(w1, w2, (__nv_bfloat16*)img, C, H, K, g.KH, g.TPS, g.KS);
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }

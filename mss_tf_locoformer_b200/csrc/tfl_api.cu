@@ -125,8 +125,8 @@ static void build_layout(tfl_plan* pl) {
       f.w1 = take((size_t)K * C * 2 * f.hidden); f.b1 = take(2 * f.hidden); f.b1raw = take(2 * f.hidden);
       f.w2 = take((size_t)K * f.hidden * C); f.b2 = take(C);
       f.tc = take(tc_ffn_image_bytes(C, f.hidden, K) / sizeof(float));
-      f.tc2_ok = tc_ffn2_image_bytes(C, f.hidden, K) > 0;
-      f.tc2 = take(tc_ffn2_image_bytes(C, f.hidden, K) / sizeof(float));
+      f.tc2_ok = tc_ffn2_image_bytes(C, f.hidden, K, c.num_groups) > 0;   // else the FFN runs on ffn_tc_kernel
+      f.tc2 = take(tc_ffn2_image_bytes(C, f.hidden, K, c.num_groups) / sizeof(float));
     }
     p.attn_gamma = take(C);
     p.rope = take(pl->head_dim / 2 + 1);
@@ -232,7 +232,7 @@ int tfl_pack_weights(const tfl_plan* pl, const float* const* w, int n_weights, v
         permute(w2, dst(f.w2), 1, K, H, C, 0, -1, (long long)C * K, K, K - 1, -1, st);
         copy(b2, f.b2, C);
         TFL_CHECK(tc_pack_ffn(w1, b1, w2, b2, (char*)packed + f.tc, C, H, K, st) == 0, "tc_pack_ffn failed");
-        if (f.tc2_ok) TFL_CHECK(tc_pack_ffn2(w1, w2, (char*)packed + f.tc2, C, H, K, st) == 0, "tc_pack_ffn2 failed");
+        if (f.tc2_ok) TFL_CHECK(tc_pack_ffn2(w1, w2, (char*)packed + f.tc2, C, H, K, c.num_groups, st) == 0, "tc_pack_ffn2 failed");
       }
       const float* attn_gamma_raw = w[i];
       copy(w[i++], p.attn_gamma, C);
@@ -583,6 +583,11 @@ extern "C" {
 int tfl_enc_conv_gln(const tfl_plan* pl, const void* packed, const float* spec, int B, int Tf, int F, float* x,
                      void* workspace, size_t ws_bytes, tfl_stream_t stream) {
   return enc_conv_gln_any(pl, packed, spec, B, Tf, F, x, workspace, ws_bytes, TFL_PRECISION_FP32, stream);
+}
+int tfl_enc_conv_gln_mode(const tfl_plan* pl, const void* packed, const float* spec, int B, int Tf, int F, float* x,
+                          void* workspace, size_t ws_bytes, int precision, tfl_stream_t stream) {
+  TFL_CHECK(precision == TFL_PRECISION_FP32 || precision == TFL_PRECISION_BF16, "unknown precision %d", precision);
+  return enc_conv_gln_any(pl, packed, spec, B, Tf, F, x, workspace, ws_bytes, precision, stream);
 }
 }  // extern "C"
 namespace tfl {

@@ -184,14 +184,15 @@ class Engine:
                                          n_samples, audio.data_ptr(), _stream()))
         return audio
 
-    def enc_conv_gln(self, spec_ri: torch.Tensor) -> torch.Tensor:
+    def enc_conv_gln(self, spec_ri: torch.Tensor, precision: int = 0) -> torch.Tensor:
+        """spec_ri [B, Tf, F, 2] -> x [B, Tf, F, C]; ``precision`` 1 is the tf32 encoder of the bf16 mode."""
         _require_cuda(spec_ri, "spec")
         B, Tf, F, _ = spec_ri.shape
         x = torch.empty((B, Tf, F, self.cfg["emb_dim"]), dtype=torch.float32, device=spec_ri.device)
         ws = self.workspace(B, Tf, F, 0, x.device)
         with torch.cuda.device(x.device):
-            check(self.lib.tfl_enc_conv_gln(self.plan, self.packed.data_ptr(), spec_ri.contiguous().data_ptr(), B, Tf,
-                                            F, x.data_ptr(), ws.data_ptr(), ws.numel(), _stream()))
+            check(self.lib.tfl_enc_conv_gln_mode(self.plan, self.packed.data_ptr(), spec_ri.contiguous().data_ptr(), B,
+                                                 Tf, F, x.data_ptr(), ws.data_ptr(), ws.numel(), precision, _stream()))
         return x
 
     def dec_conv(self, x: torch.Tensor, precision: int = 0) -> torch.Tensor:
