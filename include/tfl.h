@@ -165,6 +165,26 @@ int tfl_conv_swiglu_ffn_bwd(const tfl_plan* plan, const void* packed, const floa
 int tfl_rope_attn_bwd(const tfl_plan* plan, const void* packed, const float* const* weights, int n_weights, int layer,
                       int axis, const float* x_in, float* dx, int batch, int n_frames, int n_freq, float* grads,
                       void* workspace, size_t ws_bytes, tfl_stream_t stream);
+/* ---- autograd of the separators: a forward that keeps its activations, and its backward from an upstream gradient ----
+ * Arithmetic = TFL_OPT_TRAIN_MODE, exactly as in tfl_train_forward_backward.  The workspace of one saved forward (sub-block
+ * inputs x_0 .. x_n_sub plus the dx, scratch and weight-gradient buffers of the backward) must stay untouched between a
+ * forward and its backward; a caller that keeps several forwards alive gives each its own workspace. */
+size_t tfl_sep_train_workspace_bytes(const tfl_plan* plan, int batch, int n_frames, int n_freq);
+/* TFLocoformerSeparator (plan with enc_in_ch == 2): spec [B, Tf, F, 2] -> est [B, S, Tf, F, 2]. */
+int tfl_sep_train_forward(const tfl_plan* plan, const void* packed, const float* spec, int batch, int n_frames,
+                          int n_freq, float* est, void* workspace, size_t ws_bytes, tfl_stream_t stream);
+/* d_est [B, S, Tf, F, 2] (+ the forward's spec, packed image and workspace) -> grads (tfl_train_grad_layout,
+ * overwritten).  `weights`: the raw fp32 device tensors tfl_pack_weights took.  No gradient for spec. */
+int tfl_sep_train_backward(const tfl_plan* plan, const void* packed, const float* const* weights, int n_weights,
+                           const float* d_est, const float* spec, int batch, int n_frames, int n_freq, float* grads,
+                           void* workspace, size_t ws_bytes, tfl_stream_t stream);
+/* Blocks-only plan (enc_in_ch == 0): x_in [B, Tf, F, C] -> x_out (all Locoformer blocks); backward: dx_out -> dx_in and
+ * grads (overwritten).  x_in / x_out and dx_out / dx_in may not overlap. */
+int tfl_blocks_train_forward(const tfl_plan* plan, const void* packed, const float* x_in, int batch, int n_frames,
+                             int n_freq, float* x_out, void* workspace, size_t ws_bytes, tfl_stream_t stream);
+int tfl_blocks_train_backward(const tfl_plan* plan, const void* packed, const float* const* weights, int n_weights,
+                              const float* dx_out, int batch, int n_frames, int n_freq, float* dx_in, float* grads,
+                              void* workspace, size_t ws_bytes, tfl_stream_t stream);
 /* torch.nn.utils.clip_grad_norm_ (train.py:141): norm_out[0] = total L2 norm, norm_out[1] = min(1, max_norm / (norm + 1e-6))
  * (device, 2 floats; no host sync).  scratch: >= 592 doubles. */
 int tfl_grad_clip_norm(const float* grads, int64_t n, float max_norm, float* norm_out, double* scratch,
@@ -193,6 +213,24 @@ int tfl_bs_band_split(const float* spec, int batch, int n_chan, int n_frames, in
 int tfl_bs_band_decode(const float* x, const float* spec, int batch, int n_chan, int n_frames, int n_freq, int emb_dim,
                        int n_bands, int n_src, const int64_t* table, const float* weights, float* est, int masking,
                        tfl_stream_t stream);
+
+/* Backward of the two band stages (autograd of BSLocoformerSeparator), fp32 CUDA cores.  `d_weights` is laid out like
+ * `weights` (same table offsets, the conv weights transposed as there); each call overwrites the entries of its stage.
+ * Weight gradients are dense products over the B * T rows of a band, one CTA per output tile (deterministic).
+ * workspace: >= tfl_bs_band_bwd_workspace_bytes. */
+size_t tfl_bs_band_bwd_workspace_bytes(int batch, int n_chan, int n_frames, int n_freq, int emb_dim, int n_bands,
+                                       int n_src, int max_width);
+/* x [B, T, nb, C] (the decoder's input), spec, d_est [B, S, M, T, F, 2] -> dx [B, T, nb, C] and the gradients of table
+ * entries 6..13 (GroupNorm w / b, W1^T / b1, W3^T / b3, W4^T / b4).  The forward is recomputed per (band, frame tile). */
+int tfl_bs_band_decode_bwd(const float* x, const float* spec, const float* d_est, int batch, int n_chan, int n_frames,
+                           int n_freq, int emb_dim, int n_bands, int n_src, int max_width, const int64_t* table,
+                           const float* weights, int masking, float* dx, float* d_weights, void* workspace,
+                           size_t ws_bytes, tfl_stream_t stream);
+/* spec, dx [B, T, nb, C] (gradient of the band-split output) -> gradients of table entries 2..5 (GroupNorm(1, K_b) w / b,
+ * conv^T / bias).  No input gradient. */
+int tfl_bs_band_split_bwd(const float* spec, const float* dx, int batch, int n_chan, int n_frames, int n_freq, int emb_dim,
+                          int n_bands, int max_width, const int64_t* table, const float* weights, float* d_weights,
+                          void* workspace, size_t ws_bytes, tfl_stream_t stream);
 
 /* Diagnostic: process-wide switches used for A/B measurements (not part of the reference-facing surface).
  *   TFL_OPT_ATTN_KERNEL  1 = attn_tc_kernel (P through shared memory), 2 = attn_tc2_kernel (P in TMEM; default)

@@ -51,13 +51,21 @@ SIGNATURES = {  # name -> (restype, argtypes); must list every symbol of include
     "tfl_pair_stats": (_I, [_P, _P, _I, _L, _P, _P, _Z, _P]),
     "tfl_bs_band_split": (_I, [_P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P, _P]),
     "tfl_bs_band_decode": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P, _I, _P]),
-    "tfl_train_grad_layout": (_L, [_P, C.POINTER(_L), C.POINTER(_L), _I]),
+    "tfl_bs_band_bwd_workspace_bytes": (_Z, [_I, _I, _I, _I, _I, _I, _I, _I]),
+    "tfl_bs_band_decode_bwd": (_I, [_P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P, _I, _P, _P, _P, _Z, _P]),
+    "tfl_bs_band_split_bwd": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P, _P, _Z, _P]),
+    "tfl_train_grad_layout":(_L, [_P, C.POINTER(_L), C.POINTER(_L), _I]),
     "tfl_train_workspace_bytes": (_Z, [_P, _I, _I, _I, _I]),
     "tfl_train_stage_workspace_bytes": (_Z, [_P, _I, _I, _I]),
     "tfl_train_forward_backward": (_I, [_P, _P, C.POINTER(_P), _I, _P, _P, _I, _I, C.POINTER(TflLossConfig), _P, _P, _P, _P, _Z, _P]),
     "tfl_conv_swiglu_ffn_bwd": (_I, [_P, _P, C.POINTER(_P), _I, _I, _I, _I, _P, _P, _I, _I, _I, _P, _P, _Z, _P]),
     "tfl_rope_attn_bwd": (_I, [_P, _P, C.POINTER(_P), _I, _I, _I, _P, _P, _I, _I, _I, _P, _P, _Z, _P]),
-    "tfl_grad_clip_norm": (_I, [_P, _L, _F, _P, _P, _Z, _P]),
+    "tfl_sep_train_workspace_bytes": (_Z, [_P, _I, _I, _I]),
+    "tfl_sep_train_forward": (_I, [_P, _P, _P, _I, _I, _I, _P, _P, _Z, _P]),
+    "tfl_sep_train_backward": (_I, [_P, _P, C.POINTER(_P), _I, _P, _P, _I, _I, _I, _P, _P, _Z, _P]),
+    "tfl_blocks_train_forward": (_I, [_P, _P, _P, _I, _I, _I, _P, _P, _Z, _P]),
+    "tfl_blocks_train_backward": (_I, [_P, _P, C.POINTER(_P), _I, _P, _I, _I, _I, _P, _P, _P, _Z, _P]),
+    "tfl_grad_clip_norm":(_I, [_P, _L, _F, _P, _P, _Z, _P]),
     "tfl_grad_accumulate": (_I, [_P, _P, _L, _F, _I, _P]),
     "tfl_adamw_step": (_I, [_P, _P, _P, _P, _L, _P, _F, _F, _F, _F, _F, _I, _P]),
     "tfl_debug_set_option": (_I, [_I, _I]),

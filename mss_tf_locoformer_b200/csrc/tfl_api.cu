@@ -886,6 +886,128 @@ int tfl_bs_band_decode(const float* x, const float* spec, int B, int M, int T, i
   return 0;
 }
 
+}  // extern "C"
+namespace tfl {
+struct BsBwdWs { size_t xn, h1, h2, dh1, dh2, dxn, dz, xs, xsn, dyin, stats, sums, total; };
+static BsBwdWs bs_bwd_ws(int B, int M, int T, int F, int C, int nb, int S) {
+  BsBwdWs w{};
+  size_t off = 0;
+  auto take = [&](size_t floats) { size_t o = off; off = align_up(off + floats * sizeof(float)); return o; };
+  const size_t R = (size_t)B * T, rc = (size_t)nb * R * C;
+  w.xn = take(rc); w.h1 = take(4 * rc); w.h2 = take(4 * rc); w.dh1 = take(4 * rc); w.dh2 = take(4 * rc); w.dxn = take(rc);
+  w.dz = take(R * F * S * 4 * M);
+  w.xs = take(R * F * 2 * M); w.xsn = take(R * F * 2 * M); w.dyin = take(R * F * 2 * M);
+  w.stats = take((size_t)B * nb * 2);
+  w.sums = take((size_t)B * nb * 4);   // doubles
+  w.total = off;
+  return w;
+}
+static inline BandMat band_mat(const void* p, long long per_band, long long per_bin, int ld0, int ldw) {
+  return BandMat{(const float*)p, per_band, per_bin, ld0, ldw};
+}
+static int bs_bwd_check(int B, int M, int T, int F, int C, int nb, int S, int max_width, size_t ws_bytes) {
+  TFL_CHECK(B >= 1 && (M == 1 || M == 2) && T >= 1 && F >= 1 && C >= 1 && nb >= 1 && S >= 1 && max_width >= 1,
+            "bad band backward shape");
+  TFL_CHECK(ws_bytes >= bs_bwd_ws(B, M, T, F, C, nb, S).total, "workspace too small (%zu < %zu)", ws_bytes,
+            bs_bwd_ws(B, M, T, F, C, nb, S).total);
+  return 0;
+}
+}  // namespace tfl
+extern "C" {
+
+size_t tfl_bs_band_bwd_workspace_bytes(int B, int M, int T, int F, int C, int nb, int n_src, int max_width) {
+  (void)max_width;
+  return bs_bwd_ws(B, M, T, F, C, nb, n_src).total;
+}
+
+int tfl_bs_band_decode_bwd(const float* x, const float* spec, const float* d_est, int B, int M, int T, int F, int C, int nb,
+                           int n_src, int max_width, const int64_t* table, const float* weights, int masking, float* dx,
+                           float* d_weights, void* workspace, size_t ws_bytes, tfl_stream_t stream) {
+  NvtxRange nvtx_range("tfl::bs_band_decode_bwd");
+  TFL_CHECK(x && spec && d_est && table && weights && dx && d_weights && workspace, "null argument");
+  if (bs_bwd_check(B, M, T, F, C, nb, n_src, max_width, ws_bytes)) return -1;
+  const BsBwdWs ws = bs_bwd_ws(B, M, T, F, C, nb, n_src);
+  char* wsp = (char*)workspace;
+  cudaStream_t st = (cudaStream_t)stream;
+  const long long* tab = (const long long*)table;
+  const long long R = (long long)B * T;
+  const int C4 = 4 * C, S4M = n_src * 4 * M;
+  const size_t smem = ((size_t)9 * C * BS_TT + 64) * sizeof(float);
+  TFL_CHECK(smem <= (size_t)TC_SMEM_MAX, "emb_dim too large for the band decoder");
+  TFL_CUDA(opt_in_smem(bs_decode_bwd_rows_kernel, smem));
+  bs_decode_bwd_rows_kernel<<<dim3(nb, (T + BS_TT - 1) / BS_TT, B), 256, smem, st>>>(
+      x, spec, d_est, M, T, F, C, nb, n_src, tab, weights, masking, 1e-5f, (float*)(wsp + ws.xn), (float*)(wsp + ws.h1),
+      (float*)(wsp + ws.h2), (float*)(wsp + ws.dz));
+  TFL_LAUNCH_CHECK();
+  const BandMat xn = band_mat(wsp + ws.xn, R * C, 0, C, 0), dxn = band_mat(wsp + ws.dxn, R * C, 0, C, 0);
+  const BandMat h1 = band_mat(wsp + ws.h1, R * C4, 0, C4, 0), h2 = band_mat(wsp + ws.h2, R * C4, 0, C4, 0);
+  const BandMat dh1 = band_mat(wsp + ws.dh1, R * C4, 0, C4, 0), dh2 = band_mat(wsp + ws.dh2, R * C4, 0, C4, 0);
+  const BandMat dz = band_mat(wsp + ws.dz, 0, R * S4M, 0, S4M), none = band_mat(nullptr, 0, 0, 0, 0);
+  const unsigned rt = (unsigned)((R + 63) / 64), omax_t = (unsigned)((max_width * S4M + 63) / 64);
+  const unsigned c4_t = (unsigned)((C4 + 63) / 64), c_t = (unsigned)((C + 63) / 64);
+  // data gradients: dh2 = dz . W4, dh1 = (dh2 . W3) * tanh', dxn = dh1 . W1
+  bs_gemm_nt_kernel<<<dim3(rt, c4_t, nb), 256, 0, st>>>(BsGemm{dz, dh2, none, C4, 0, 0, S4M, 12, R}, tab, weights);
+  TFL_LAUNCH_CHECK();
+  bs_gemm_nt_kernel<<<dim3(rt, c4_t, nb), 256, 0, st>>>(BsGemm{dh2, dh1, h1, C4, 0, C4, 0, 10, R}, tab, weights);
+  TFL_LAUNCH_CHECK();
+  bs_gemm_nt_kernel<<<dim3(rt, c_t, nb), 256, 0, st>>>(BsGemm{dh1, dxn, none, C, 0, C4, 0, 8, R}, tab, weights);
+  TFL_LAUNCH_CHECK();
+  // weight and bias gradients of the three 1x1 convs
+  bs_wgrad_kernel<<<dim3(omax_t, c4_t, nb), 256, 0, st>>>(BsWgrad{h2, dz, C4, 0, 0, S4M, 12, 13, R}, tab, d_weights);
+  TFL_LAUNCH_CHECK();
+  bs_wgrad_kernel<<<dim3(c4_t, c4_t, nb), 256, 0, st>>>(BsWgrad{h1, dh2, C4, 0, C4, 0, 10, 11, R}, tab, d_weights);
+  TFL_LAUNCH_CHECK();
+  bs_wgrad_kernel<<<dim3(c4_t, c_t, nb), 256, 0, st>>>(BsWgrad{xn, dh1, C, 0, C4, 0, 8, 9, R}, tab, d_weights);
+  TFL_LAUNCH_CHECK();
+  // GroupNorm(1, C) over (C, T): statistics and the two sums, then its parameter gradients and dx
+  const BsNorm nrm{band_mat(x, C, 0, nb * C, 0), dxn, C, 0, 6, T};
+  float* stats = (float*)(wsp + ws.stats);
+  double* sums = (double*)(wsp + ws.sums);
+  bs_gn_sums_kernel<<<dim3(nb, B), 256, 0, st>>>(nrm, tab, weights, 1e-5f, stats, sums);
+  TFL_LAUNCH_CHECK();
+  bs_gn_bwd_kernel<<<dim3(nb, (C + 31) / 32), dim3(32, 8), 0, st>>>(nrm, band_mat(dx, C, 0, nb * C, 0), B, tab, weights,
+                                                                    stats, sums, d_weights);
+  TFL_LAUNCH_CHECK();
+  return 0;
+}
+
+int tfl_bs_band_split_bwd(const float* spec, const float* dx, int B, int M, int T, int F, int C, int nb, int max_width,
+                          const int64_t* table, const float* weights, float* d_weights, void* workspace, size_t ws_bytes,
+                          tfl_stream_t stream) {
+  NvtxRange nvtx_range("tfl::bs_band_split_bwd");
+  TFL_CHECK(spec && dx && table && weights && d_weights && workspace, "null argument");
+  if (bs_bwd_check(B, M, T, F, C, nb, 1, max_width, ws_bytes)) return -1;
+  const BsBwdWs ws = bs_bwd_ws(B, M, T, F, C, nb, 1);
+  char* wsp = (char*)workspace;
+  cudaStream_t st = (cudaStream_t)stream;
+  const long long* tab = (const long long*)table;
+  const long long R = (long long)B * T;
+  const int M2 = 2 * M;
+  float* stats = (float*)(wsp + ws.stats);
+  const BandMat xs = band_mat(wsp + ws.xs, 0, R * M2, 0, M2), xsn = band_mat(wsp + ws.xsn, 0, R * M2, 0, M2);
+  const BandMat dyin = band_mat(wsp + ws.dyin, 0, R * M2, 0, M2), dxm = band_mat(dx, C, 0, nb * C, 0);
+  const BandMat none = band_mat(nullptr, 0, 0, 0, 0);
+  // input features, their GroupNorm(1, K_b) statistics over (K_b, T), and the normalised features
+  bs_split_rows_kernel<<<dim3(nb, B), 256, 0, st>>>(spec, M, T, F, tab, weights, nullptr, (float*)(wsp + ws.xs), nullptr);
+  TFL_LAUNCH_CHECK();
+  const BsNorm nrm{xs, dyin, 0, M2, 2, T};
+  bs_gn_sums_kernel<<<dim3(nb, B), 256, 0, st>>>(BsNorm{xs, none, 0, M2, 2, T}, tab, weights, 1e-5f, stats, nullptr);
+  TFL_LAUNCH_CHECK();
+  bs_split_rows_kernel<<<dim3(nb, B), 256, 0, st>>>(spec, M, T, F, tab, weights, stats, (float*)(wsp + ws.xs),
+                                                    (float*)(wsp + ws.xsn));
+  TFL_LAUNCH_CHECK();
+  // conv weight / bias gradients, then the gradient of the GroupNorm output and its parameter gradients
+  const unsigned rt = (unsigned)((R + 63) / 64), kt = (unsigned)((max_width * M2 + 63) / 64), ct = (unsigned)((C + 63) / 64);
+  bs_wgrad_kernel<<<dim3(ct, kt, nb), 256, 0, st>>>(BsWgrad{xsn, dxm, 0, M2, C, 0, 4, 5, R}, tab, d_weights);
+  TFL_LAUNCH_CHECK();
+  bs_gemm_nt_kernel<<<dim3(rt, kt, nb), 256, 0, st>>>(BsGemm{dxm, dyin, none, 0, M2, C, 0, 4, R}, tab, weights);
+  TFL_LAUNCH_CHECK();
+  bs_gn_bwd_kernel<<<dim3(nb, (max_width * M2 + 31) / 32), dim3(32, 8), 0, st>>>(nrm, none, B, tab, weights, stats, nullptr,
+                                                                                 d_weights);
+  TFL_LAUNCH_CHECK();
+  return 0;
+}
+
 int tfl_pair_stats(const float* est, const float* tgt, int rows, int64_t n, double* out5, double* scratch,
                    size_t scratch_bytes, tfl_stream_t stream) {
   TFL_CHECK(est && tgt && out5 && scratch, "null argument");

@@ -63,20 +63,22 @@ struct TrainWs {
   int n_sub, l_frames, l_freq;
 };
 
-// (B, Tf, F) size the network buffers; T (audio samples, 0 = stage-level use) and the loss STFT size the rest
-static TrainWs plan_train_ws(const tfl_plan* pl, int B, int Tf, int F, int T, int l_fft, int l_hop) {
+// (B, Tf, F) size the network buffers; T (audio samples, 0 = stage-level use) and the loss STFT size the rest.
+// `saved` (frames-only mode, T = 0): the checkpoint slots of one saved forward without the STFT / loss buffers.
+static TrainWs plan_train_ws(const tfl_plan* pl, int B, int Tf, int F, int T, int l_fft, int l_hop, bool saved = false) {
   const tfl_config& c = pl->cfg;
   TrainWs w{};
+  const bool ckpt = T > 0 || saved;
   w.fwd = plan_workspace(pl, B, Tf, F, TFL_PRECISION_FP32);
   size_t off = align_up(w.fwd.total);
   auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes); return o; };
   const size_t N = (size_t)B * Tf * F;
   const size_t C = c.emb_dim, A = c.attention_dim, K = c.conv_kernel, S = c.n_src;
   const size_t Hmax = c.ffn_hidden0 > c.ffn_hidden1 ? c.ffn_hidden0 : c.ffn_hidden1;
-  w.n_sub = T > 0 ? c.n_layers * 2 * (pl->n_ffn + 1) : 0;
+  w.n_sub = ckpt ? c.n_layers * 2 * (pl->n_ffn + 1) : 0;
   w.ckpt = take((size_t)(w.n_sub > 0 ? w.n_sub + 1 : 0) * N * C * sizeof(float));   // x_0 .. x_n_sub (the residual stream itself)
   w.fwd16_base = 0;
-  if (T > 0 && attn_tc_supported((int)C, c.n_heads, pl->head_dim)) {
+  if (ckpt && attn_tc_supported((int)C, c.n_heads, pl->head_dim)) {
     w.fwd16 = plan_workspace(pl, B, Tf, F, TFL_PRECISION_BF16);
     w.fwd16_base = take(w.fwd16.total);
   }
@@ -357,6 +359,135 @@ static int check_train(const tfl_plan* pl, const void* packed, const float* cons
   return timeout_pending();
 }
 
+// ---- pieces of a training step, shared by the MSS step and the separator / blocks autograd entry points ----------------
+static float* ckpt_slot(const TrainWs& tw, char* wsp, Dims d, int C, size_t k) {
+  return (float*)(wsp + tw.ckpt + k * (size_t)d.B * d.Tf * d.F * C * sizeof(float));
+}
+
+// The sub-blocks with the residual stream kept: x_k = input of sub-block k lives in checkpoint slot k (slot 0 must hold
+// the blocks' input; slot n_sub receives their output).  Mixed mode (TFL_OPT_TRAIN_MODE 2, the reference's bf16-autocast
+// forward): sub-blocks the tcgen05 kernels cover run on them -- the fused FFN kernel writes slot k + 1 straight from
+// slot k --, the rest stays on the fp32 path.
+static int saved_blocks_forward(const tfl_plan* pl, const char* pk, Dims d, const TrainWs& tw, char* wsp, bool mixed,
+                                cudaStream_t st) {
+  const tfl_config& c = pl->cfg;
+  const size_t act_bytes = (size_t)d.B * d.Tf * d.F * c.emb_dim * sizeof(float);
+  const std::vector<SubBlock> subs = sub_blocks(pl);
+  for (size_t k = 0; k < subs.size(); ++k) {
+    const SubBlock& sb = subs[k];
+    float* x_in = ckpt_slot(tw, wsp, d, c.emb_dim, k);
+    float* x_out = ckpt_slot(tw, wsp, d, c.emb_dim, k + 1);
+    if (sb.kind == 2) {
+      TFL_CUDA(cudaMemcpyAsync(x_out, x_in, act_bytes, cudaMemcpyDeviceToDevice, st));
+      if (mixed && tw.fwd16_base != 0) {
+        if (attn_bf16(pl, pk, sb.layer, sb.axis, x_out, d, tw.fwd16, wsp + tw.fwd16_base, st)) return -1;
+      } else if (attn_f32(pl, pk, sb.layer, sb.axis, x_out, d, tw.fwd, wsp, st)) return -1;
+    } else {
+      const FfnPack& f = pl->lay.paths[(size_t)sb.layer * 2 + sb.axis].ffn[sb.kind];
+      FfnTcGeom geom;
+      if (mixed && ffn_tc_geometry(c.emb_dim, f.hidden, c.conv_kernel, c.num_groups, &geom)) {
+        if (tc_ffn(pl, pk, sb.layer, sb.axis, sb.kind, x_in, x_out, d.B, d.Tf, d.F, st)) return -1;
+      } else {
+        TFL_CUDA(cudaMemcpyAsync(x_out, x_in, act_bytes, cudaMemcpyDeviceToDevice, st));
+        if (ffn_f32(pl, pk, sb.layer, sb.axis, sb.kind, x_out, d, tw.fwd, wsp, st)) return -1;
+      }
+    }
+  }
+  return 0;
+}
+
+// Backward of the sub-blocks: tw.dx holds dL/d(blocks output) on entry and dL/d(blocks input) on exit; the parameter
+// gradients land in their slices of `grads` (accumulated: the caller zeroes the buffer).
+static int blocks_backward(const tfl_plan* pl, const char* pk, const float* const* w, const GradLayout& gl, float* grads,
+                           Dims d, const TrainWs& tw, char* wsp, cudaStream_t st) {
+  float* dx = (float*)(wsp + tw.dx);
+  const std::vector<SubBlock> subs = sub_blocks(pl);
+  for (int k = (int)subs.size() - 1; k >= 0; --k) {
+    const SubBlock& sb = subs[k];
+    const float* x_in = ckpt_slot(tw, wsp, d, pl->cfg.emb_dim, (size_t)k);
+    GradPtrs gp; RawPtrs rp;
+    path_ptrs(pl, gl, grads, w, sb.layer, sb.axis, gp, rp);
+    if (sb.kind == 2) { if (attn_backward(pl, pk, sb.layer, sb.axis, x_in, dx, d, tw, wsp, gp, rp, st)) return -1; }
+    else if (ffn_backward(pl, pk, sb.layer, sb.axis, sb.kind, x_in, dx, d, tw, wsp, gp, rp, st)) return -1;
+  }
+  return 0;
+}
+
+// Decoder backward from dEst [B, S, Tf, F, 2]: deconv.weight / deconv.bias gradients, and dL/dx (decoder input x) into
+// tw.dx.
+static int dec_backward(const tfl_plan* pl, const char* pk, const GradLayout& gl, float* grads, int n_w, const float* x,
+                        const float* dest, Dims d, const TrainWs& tw, char* wsp, cudaStream_t st) {
+  const int C = pl->cfg.emb_dim, S = pl->cfg.n_src;
+  const size_t N = (size_t)d.B * d.Tf * d.F;
+  const int cthreads = (C + 31) / 32 * 32;
+  float* nat = (float*)(wsp + tw.nat);
+  float* dx = (float*)(wsp + tw.dx);
+  // weights: natural layout [9][8][C] -> deconv.weight [C, 2S, 3, 3]
+  TFL_CUDA(cudaMemsetAsync(nat, 0, ((size_t)9 * 8 * C + 8) * sizeof(float), st));
+  dec_wgrad_kernel<<<pl->sm_count * 4, cthreads, 0, st>>>(x, dest, d.Tf, d.F, C, 2 * S, (long long)N, nat);
+  TFL_LAUNCH_CHECK();
+  permute(nat, grads + gl.off[n_w - 2], C, 2 * S, 3, 3, 1, C, (long long)3 * 8 * C, (long long)8 * C, 0, -1, st);
+  dec_bias_grad_kernel<<<2 * S, 256, 0, st>>>(dest, d.B, S, (long long)d.Tf * d.F, grads + gl.off[n_w - 1]);
+  TFL_LAUNCH_CHECK();
+  const size_t smem = (size_t)9 * C * 8 * sizeof(float);
+  TFL_CUDA(opt_in_smem(dec_dgrad_kernel, smem));
+  dec_dgrad_kernel<<<pl->sm_count * 8, 256, smem, st>>>(dest, d.Tf, d.F, C, 2 * S, (const float*)(pk + pl->lay.dec_w), dx,
+                                                       (long long)N);
+  TFL_LAUNCH_CHECK();
+  return 0;
+}
+
+// Encoder backward from tw.dx = dL/d(encoder output): v = conv(spec) recomputed into xn, then GroupNorm(1, C) backward
+// and the conv weight gradient.  No gradient for spec.
+static int enc_backward(const tfl_plan* pl, const char* pk, const GradLayout& gl, float* grads, const float* spec, Dims d,
+                        const TrainWs& tw, char* wsp, cudaStream_t st) {
+  const tfl_config& c = pl->cfg;
+  const int C = c.emb_dim, B = d.B, Tf = d.Tf, F = d.F;
+  const int cthreads = (C + 31) / 32 * 32;
+  float* nat = (float*)(wsp + tw.nat);
+  float* dx = (float*)(wsp + tw.dx);
+  float* v = (float*)(wsp + tw.fwd.xn);
+  double* part = (double*)(wsp + tw.fwd.gln_part);
+  float* stats = (float*)(wsp + tw.fwd.gln_stats);
+  double* sums = (double*)(wsp + tw.enc_sums);
+  const size_t smem = ((size_t)9 * 2 * C + C) * sizeof(float);
+  enc_conv_kernel<2><<<dim3(tw.fwd.gln_blocks, B), 256, smem, st>>>(spec, Tf, F, C, (const float*)(pk + pl->lay.enc_w),
+                                                                   (const float*)(pk + pl->lay.enc_b), v, part);
+  TFL_LAUNCH_CHECK();
+  gln_finalize_kernel<<<B, 256, 0, st>>>(part, tw.fwd.gln_blocks, (double)Tf * F * C, c.eps, stats);
+  TFL_LAUNCH_CHECK();
+  TFL_CUDA(cudaMemsetAsync(sums, 0, (size_t)B * 2 * sizeof(double), st));
+  TFL_CUDA(cudaMemsetAsync(nat, 0, ((size_t)18 * C + C) * sizeof(float), st));
+  enc_gln_bwd_stats_kernel<<<dim3(pl->sm_count * 2, B), cthreads, 0, st>>>(v, dx, (long long)Tf * F, C, stats, (const float*)(pk + pl->lay.gln_w),
+                                                                         grads + gl.off[2], grads + gl.off[3], sums);
+  TFL_LAUNCH_CHECK();
+  enc_wgrad_kernel<2><<<dim3(pl->sm_count * 2, B), cthreads, 0, st>>>(v, dx, spec, Tf, F, C, stats, sums, (const float*)(pk + pl->lay.gln_w),
+                                                                    nat, nat + (size_t)18 * C);
+  TFL_LAUNCH_CHECK();
+  // natural [9][ci][C] -> conv.0.weight [C, ci, 3, 3]
+  permute(nat, grads + gl.off[0], 1, C, 2, 9, 0, 1, C, (long long)2 * C, 0, -1, st);
+  permute(nat + (size_t)18 * C, grads + gl.off[1], 1, 1, 1, C, 0, 0, 0, 1, 0, -1, st);
+  TFL_LAUNCH_CHECK();
+  return 0;
+}
+
+// Shared argument checks of the saved-forward / backward pairs; fills the workspace plan.
+static int check_saved(const tfl_plan* pl, const void* packed, int B, int Tf, int F, bool conv, size_t ws_bytes, TrainWs* tw) {
+  TFL_CHECK(pl && packed, "null argument");
+  TFL_CHECK(B >= 1 && Tf >= 1 && F >= 1, "empty input (batch %d, frames %d, bins %d)", B, Tf, F);
+  TFL_CHECK(pl->cfg.emb_dim <= 256, "training kernels support emb_dim <= 256");
+  if (conv) {
+    TFL_CHECK(pl->cfg.enc_in_ch == 2, "this entry point needs a plan with the conv encoder / decoder (enc_in_ch == 2)");
+    TFL_CHECK(pl->cfg.n_src * 2 <= 8, "the decoder backward supports at most 4 sources");
+  } else {
+    TFL_CHECK(pl->cfg.enc_in_ch == 0, "this entry point needs a blocks-only plan (enc_in_ch == 0)");
+  }
+  *tw = plan_train_ws(pl, B, Tf, F, 0, 0, 0, /*saved=*/true);
+  TFL_CHECK(ws_bytes >= tw->total, "workspace too small (%zu < %zu)", ws_bytes, tw->total);
+  if (ensure_device_ready()) return -1;
+  return timeout_pending();
+}
+
 }  // namespace tfl
 
 extern "C" {
@@ -448,48 +579,23 @@ int tfl_train_forward_backward(const tfl_plan* pl, const void* packed, const flo
   char* wsp = (char*)workspace;
   const char* pk = (const char*)packed;
   const GradLayout gl = grad_layout(pl);
-  const size_t N = (size_t)B * Tf * F, act_bytes = N * C * sizeof(float);
   float* spec = (float*)(wsp + tw.fwd.spec);
   float* est = (float*)(wsp + tw.fwd.est);
   float* audio = (float*)(wsp + tw.audio);
   float* daudio = (float*)(wsp + tw.daudio);
   float* dest = (float*)(wsp + tw.dest);
-  float* dx = (float*)(wsp + tw.dx);
-  float* nat = (float*)(wsp + tw.nat);
   TFL_CUDA(cudaMemsetAsync(grads, 0, (size_t)gl.total * sizeof(float), st));
 
   // ---------------- forward ----------------
-  // The residual stream is kept: x_k = input of sub-block k lives in checkpoint slot k (x_0 = encoder output, x_n_sub =
-  // decoder input).  Mixed mode (TFL_OPT_TRAIN_MODE 2, the reference's bf16-autocast forward): sub-blocks the tcgen05
-  // kernels cover run on them -- the fused FFN kernel writes slot k + 1 straight from slot k --, the rest and the whole
-  // backward pass stay on the tf32 / fp32 GEMM path.
+  // The residual stream is kept (saved_blocks_forward): x_0 = encoder output, x_n_sub = decoder input.  Mixed mode runs
+  // the encoder / decoder in the tf32 arithmetic of the bf16 inference path; the whole backward pass stays on the tf32 /
+  // fp32 GEMM path.
   const bool mixed = tfl_option(TFL_OPT_TRAIN_MODE) >= 2;
   const int enc_prec = mixed ? TFL_PRECISION_BF16 : TFL_PRECISION_FP32;
-  auto slot = [&](size_t k) { return (float*)(wsp + tw.ckpt + k * act_bytes); };
   if (tfl_stft(pl, packed, mixture, B, T, spec, stream)) return -1;
-  if (enc_conv_gln_any(pl, packed, spec, B, Tf, F, slot(0), workspace, ws_bytes, enc_prec, stream)) return -1;
-  const std::vector<SubBlock> subs = sub_blocks(pl);
-  for (size_t k = 0; k < subs.size(); ++k) {
-    const SubBlock& sb = subs[k];
-    float* x_in = slot(k);
-    float* x_out = slot(k + 1);
-    if (sb.kind == 2) {
-      TFL_CUDA(cudaMemcpyAsync(x_out, x_in, act_bytes, cudaMemcpyDeviceToDevice, st));
-      if (mixed && tw.fwd16_base != 0) {
-        if (attn_bf16(pl, pk, sb.layer, sb.axis, x_out, d, tw.fwd16, wsp + tw.fwd16_base, st)) return -1;
-      } else if (attn_f32(pl, pk, sb.layer, sb.axis, x_out, d, tw.fwd, wsp, st)) return -1;
-    } else {
-      const FfnPack& f = pl->lay.paths[(size_t)sb.layer * 2 + sb.axis].ffn[sb.kind];
-      FfnTcGeom geom;
-      if (mixed && ffn_tc_geometry(c.emb_dim, f.hidden, c.conv_kernel, c.num_groups, &geom)) {
-        if (tc_ffn(pl, pk, sb.layer, sb.axis, sb.kind, x_in, x_out, B, Tf, F, st)) return -1;
-      } else {
-        TFL_CUDA(cudaMemcpyAsync(x_out, x_in, act_bytes, cudaMemcpyDeviceToDevice, st));
-        if (ffn_f32(pl, pk, sb.layer, sb.axis, sb.kind, x_out, d, tw.fwd, wsp, st)) return -1;
-      }
-    }
-  }
-  float* x = slot(subs.size());                                  // decoder input
+  if (enc_conv_gln_any(pl, packed, spec, B, Tf, F, ckpt_slot(tw, wsp, d, C, 0), workspace, ws_bytes, enc_prec, stream)) return -1;
+  if (saved_blocks_forward(pl, pk, d, tw, wsp, mixed, st)) return -1;
+  const float* x = ckpt_slot(tw, wsp, d, C, (size_t)tw.n_sub);   // decoder input
   if (dec_conv_any(pl, packed, x, B, Tf, F, est, enc_prec, stream)) return -1;
   if (tfl_istft_ola(pl, packed, est, B, Tf, T, audio, stream)) return -1;
   if (est_audio != nullptr)
@@ -546,52 +652,96 @@ int tfl_train_forward_backward(const tfl_plan* pl, const void* packed, const flo
                                                        (const float2*)(pk + pl->lay.twiddle), (const float*)(pk + pl->lay.window), dest);
     TFL_LAUNCH_CHECK();
   }
-  const int n_w = n_weights;
-  const int cthreads = (C + 31) / 32 * 32;
-  {   // decoder: weights (natural layout [9][8][C] -> deconv.weight [C, 2S, 3, 3]) and data
-    TFL_CUDA(cudaMemsetAsync(nat, 0, ((size_t)9 * 8 * C + 8) * sizeof(float), st));
-    dec_wgrad_kernel<<<pl->sm_count * 4, cthreads, 0, st>>>(x, dest, Tf, F, C, 2 * S, (long long)N, nat);
-    TFL_LAUNCH_CHECK();
-    permute(nat, grads + gl.off[n_w - 2], C, 2 * S, 3, 3, 1, C, (long long)3 * 8 * C, (long long)8 * C, 0, -1, st);
-    dec_bias_grad_kernel<<<2 * S, 256, 0, st>>>(dest, B, S, (long long)Tf * F, grads + gl.off[n_w - 1]);
-    TFL_LAUNCH_CHECK();
-    const size_t smem = (size_t)9 * C * 8 * sizeof(float);
-    TFL_CUDA(opt_in_smem(dec_dgrad_kernel, smem));
-    dec_dgrad_kernel<<<pl->sm_count * 8, 256, smem, st>>>(dest, Tf, F, C, 2 * S, (const float*)(pk + pl->lay.dec_w), dx, (long long)N);
-    TFL_LAUNCH_CHECK();
-  }
-  for (int k = (int)subs.size() - 1; k >= 0; --k) {
-    const SubBlock& sb = subs[k];
-    const float* x_in = (const float*)(wsp + tw.ckpt + (size_t)k * act_bytes);
-    GradPtrs gp; RawPtrs rp;
-    path_ptrs(pl, gl, grads, w, sb.layer, sb.axis, gp, rp);
-    if (sb.kind == 2) { if (attn_backward(pl, pk, sb.layer, sb.axis, x_in, dx, d, tw, wsp, gp, rp, st)) return -1; }
-    else if (ffn_backward(pl, pk, sb.layer, sb.axis, sb.kind, x_in, dx, d, tw, wsp, gp, rp, st)) return -1;
-  }
-  {   // encoder: v = conv(spec) recomputed into xn, then GroupNorm(1, C) backward and the conv weight gradient
-    float* v = (float*)(wsp + tw.fwd.xn);
-    double* part = (double*)(wsp + tw.fwd.gln_part);
-    float* stats = (float*)(wsp + tw.fwd.gln_stats);
-    double* sums = (double*)(wsp + tw.enc_sums);
-    const size_t smem = ((size_t)9 * 2 * C + C) * sizeof(float);
-    enc_conv_kernel<2><<<dim3(tw.fwd.gln_blocks, B), 256, smem, st>>>(spec, Tf, F, C, (const float*)(pk + pl->lay.enc_w),
-                                                                     (const float*)(pk + pl->lay.enc_b), v, part);
-    TFL_LAUNCH_CHECK();
-    gln_finalize_kernel<<<B, 256, 0, st>>>(part, tw.fwd.gln_blocks, (double)Tf * F * C, c.eps, stats);
-    TFL_LAUNCH_CHECK();
-    TFL_CUDA(cudaMemsetAsync(sums, 0, (size_t)B * 2 * sizeof(double), st));
-    TFL_CUDA(cudaMemsetAsync(nat, 0, ((size_t)18 * C + C) * sizeof(float), st));
-    enc_gln_bwd_stats_kernel<<<dim3(pl->sm_count * 2, B), cthreads, 0, st>>>(v, dx, (long long)Tf * F, C, stats, (const float*)(pk + pl->lay.gln_w),
-                                                                           grads + gl.off[2], grads + gl.off[3], sums);
-    TFL_LAUNCH_CHECK();
-    enc_wgrad_kernel<2><<<dim3(pl->sm_count * 2, B), cthreads, 0, st>>>(v, dx, spec, Tf, F, C, stats, sums, (const float*)(pk + pl->lay.gln_w),
-                                                                      nat, nat + (size_t)18 * C);
-    TFL_LAUNCH_CHECK();
-    // natural [9][ci][C] -> conv.0.weight [C, ci, 3, 3]
-    permute(nat, grads + gl.off[0], 1, C, 2, 9, 0, 1, C, (long long)2 * C, 0, -1, st);
-    permute(nat + (size_t)18 * C, grads + gl.off[1], 1, 1, 1, C, 0, 0, 0, 1, 0, -1, st);
-    TFL_LAUNCH_CHECK();
-  }
+  if (dec_backward(pl, pk, gl, grads, n_weights, x, dest, d, tw, wsp, st)) return -1;
+  if (blocks_backward(pl, pk, w, gl, grads, d, tw, wsp, st)) return -1;
+  return enc_backward(pl, pk, gl, grads, spec, d, tw, wsp, st);
+}
+
+size_t tfl_sep_train_workspace_bytes(const tfl_plan* pl, int B, int Tf, int F) {
+  return pl == nullptr ? 0 : plan_train_ws(pl, B, Tf, F, 0, 0, 0, /*saved=*/true).total;
+}
+
+// TFLocoformerSeparator forward with the sub-block inputs saved in `workspace` for tfl_sep_train_backward: the stages of
+// tfl_separator_forward in the arithmetic the MSS training step uses for TFL_OPT_TRAIN_MODE.
+int tfl_sep_train_forward(const tfl_plan* pl, const void* packed, const float* spec, int B, int Tf, int F, float* est,
+                          void* workspace, size_t ws_bytes, tfl_stream_t stream) {
+  NvtxRange nvtx_range("tfl::sep_train_forward");
+  Tf32Scope tf32_scope;
+  TrainWs tw;
+  if (check_saved(pl, packed, B, Tf, F, true, ws_bytes, &tw)) return -1;
+  TFL_CHECK(spec && est && workspace, "null argument");
+  const Dims d{B, Tf, F};
+  const bool mixed = tfl_option(TFL_OPT_TRAIN_MODE) >= 2;
+  const int prec = mixed ? TFL_PRECISION_BF16 : TFL_PRECISION_FP32;
+  char* wsp = (char*)workspace;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (enc_conv_gln_any(pl, packed, spec, B, Tf, F, ckpt_slot(tw, wsp, d, pl->cfg.emb_dim, 0), workspace, ws_bytes, prec,
+                       stream)) return -1;
+  if (saved_blocks_forward(pl, (const char*)packed, d, tw, wsp, mixed, st)) return -1;
+  return dec_conv_any(pl, packed, ckpt_slot(tw, wsp, d, pl->cfg.emb_dim, (size_t)tw.n_sub), B, Tf, F, est, prec, stream);
+}
+
+// Backward of tfl_sep_train_forward from dEst [B, S, Tf, F, 2] (same spec, packed image and workspace as the forward):
+// every parameter gradient into `grads` (tfl_train_grad_layout, overwritten).  No gradient for spec.
+int tfl_sep_train_backward(const tfl_plan* pl, const void* packed, const float* const* w, int n_weights, const float* d_est,
+                           const float* spec, int B, int Tf, int F, float* grads, void* workspace, size_t ws_bytes,
+                           tfl_stream_t stream) {
+  NvtxRange nvtx_range("tfl::sep_train_backward");
+  Tf32Scope tf32_scope;
+  if (check_train(pl, packed, w, n_weights)) return -1;
+  TrainWs tw;
+  if (check_saved(pl, packed, B, Tf, F, true, ws_bytes, &tw)) return -1;
+  TFL_CHECK(d_est && spec && grads && workspace, "null argument");
+  const Dims d{B, Tf, F};
+  const char* pk = (const char*)packed;
+  char* wsp = (char*)workspace;
+  cudaStream_t st = (cudaStream_t)stream;
+  const GradLayout gl = grad_layout(pl);
+  TFL_CUDA(cudaMemsetAsync(grads, 0, (size_t)gl.total * sizeof(float), st));
+  const float* x = ckpt_slot(tw, wsp, d, pl->cfg.emb_dim, (size_t)tw.n_sub);
+  if (dec_backward(pl, pk, gl, grads, n_weights, x, d_est, d, tw, wsp, st)) return -1;
+  if (blocks_backward(pl, pk, w, gl, grads, d, tw, wsp, st)) return -1;
+  return enc_backward(pl, pk, gl, grads, spec, d, tw, wsp, st);
+}
+
+// The same pair for a blocks-only plan (enc_in_ch == 0): x_in [B, Tf, F, C] -> x_out, and from dL/dx_out the block
+// parameter gradients and dL/dx_in.  Tf / F are the two sequence axes (BS-Locoformer: frames and bands).
+int tfl_blocks_train_forward(const tfl_plan* pl, const void* packed, const float* x_in, int B, int Tf, int F, float* x_out,
+                             void* workspace, size_t ws_bytes, tfl_stream_t stream) {
+  NvtxRange nvtx_range("tfl::blocks_train_forward");
+  Tf32Scope tf32_scope;
+  TrainWs tw;
+  if (check_saved(pl, packed, B, Tf, F, false, ws_bytes, &tw)) return -1;
+  TFL_CHECK(x_in && x_out && workspace, "null argument");
+  const Dims d{B, Tf, F};
+  const int C = pl->cfg.emb_dim;
+  const size_t act_bytes = (size_t)B * Tf * F * C * sizeof(float);
+  char* wsp = (char*)workspace;
+  cudaStream_t st = (cudaStream_t)stream;
+  TFL_CUDA(cudaMemcpyAsync(ckpt_slot(tw, wsp, d, C, 0), x_in, act_bytes, cudaMemcpyDeviceToDevice, st));
+  if (saved_blocks_forward(pl, (const char*)packed, d, tw, wsp, tfl_option(TFL_OPT_TRAIN_MODE) >= 2, st)) return -1;
+  TFL_CUDA(cudaMemcpyAsync(x_out, ckpt_slot(tw, wsp, d, C, (size_t)tw.n_sub), act_bytes, cudaMemcpyDeviceToDevice, st));
+  return 0;
+}
+
+int tfl_blocks_train_backward(const tfl_plan* pl, const void* packed, const float* const* w, int n_weights,
+                              const float* dx_out, int B, int Tf, int F, float* dx_in, float* grads, void* workspace,
+                              size_t ws_bytes, tfl_stream_t stream) {
+  NvtxRange nvtx_range("tfl::blocks_train_backward");
+  Tf32Scope tf32_scope;
+  if (check_train(pl, packed, w, n_weights)) return -1;
+  TrainWs tw;
+  if (check_saved(pl, packed, B, Tf, F, false, ws_bytes, &tw)) return -1;
+  TFL_CHECK(dx_out && dx_in && grads && workspace, "null argument");
+  const Dims d{B, Tf, F};
+  const size_t act_bytes = (size_t)B * Tf * F * pl->cfg.emb_dim * sizeof(float);
+  char* wsp = (char*)workspace;
+  cudaStream_t st = (cudaStream_t)stream;
+  const GradLayout gl = grad_layout(pl);
+  TFL_CUDA(cudaMemsetAsync(grads, 0, (size_t)gl.total * sizeof(float), st));
+  TFL_CUDA(cudaMemcpyAsync(wsp + tw.dx, dx_out, act_bytes, cudaMemcpyDeviceToDevice, st));
+  if (blocks_backward(pl, (const char*)packed, w, gl, grads, d, tw, wsp, st)) return -1;
+  TFL_CUDA(cudaMemcpyAsync(dx_in, wsp + tw.dx, act_bytes, cudaMemcpyDeviceToDevice, st));
   return 0;
 }
 

@@ -29,13 +29,16 @@ class TFLocoformerSeparator(_Standalone, _Base):
                  norm_type: str = "rmsgrouporm", num_groups: int = 4, tf_order: str = "ft", n_heads: int = 4,
                  flash_attention: bool = False, attention_dim: int = 128, pos_enc: str = "rope",
                  ffn_type: Union[str, list] = "swiglu_conv1d", ffn_hidden_dim: Union[int, list] = 384,
-                 conv1d_kernel: int = 4, conv1d_shift: int = 1, dropout: float = 0.0, eps: float = 1.0e-5):
-        # input_dim is accepted and unused, as in the reference (:66-89)
+                 conv1d_kernel: int = 4, conv1d_shift: int = 1, dropout: float = 0.0, eps: float = 1.0e-5,
+                 differentiable: bool = False):
+        # input_dim is accepted and unused, as in the reference (:66-89).  differentiable (not in the reference; an
+        # ESPnet separator_conf key): train through torch autograd -- ESPnet's own loss, DDP and optimiser (autograd.py)
         _Standalone.__init__(self, num_spk=num_spk, n_layers=n_layers, emb_dim=emb_dim, norm_type=norm_type,
                              num_groups=num_groups, tf_order=tf_order, n_heads=n_heads, flash_attention=flash_attention,
                              attention_dim=attention_dim, pos_enc=pos_enc, ffn_type=ffn_type,
                              ffn_hidden_dim=ffn_hidden_dim, conv1d_kernel=conv1d_kernel, conv1d_shift=conv1d_shift,
                              dropout=dropout, eps=eps)
+        self.differentiable = bool(differentiable)
 
     def forward(self, input: torch.Tensor, ilens: torch.Tensor, additional: Optional[Dict] = None
                 ) -> Tuple[List[torch.Tensor], torch.Tensor, OrderedDict]:

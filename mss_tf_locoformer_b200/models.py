@@ -6,6 +6,8 @@ import torch
 import torch.nn as nn
 
 from .engine import Engine
+from .autograd import BSFunction, SeparatorFunction, bs_band_params, wants_autograd
+from .engine import _require_cuda
 from .modules import (MSSTransform, RotaryEmbedding, TFLocoformerBlock, SOURCE_NAMES, _forward_only,
                       _resolve_precision)
 
@@ -14,6 +16,9 @@ class _SeparatorBase(nn.Module):
     """Shared plumbing: engine creation, lazy weight packing, sub-module call sites."""
 
     precision: Optional[str] = None  # None = follow torch.autocast (bf16) else fp32; or "fp32" / "bf16"
+    # True: in training mode with grad enabled, forward builds an autograd graph over the parameters (autograd.py;
+    # TFLocoformerSeparator and BSLocoformerSeparator).  TFLocoformerMSS trains through training.Trainer instead.
+    differentiable: bool = False
 
     def _init_engine_cfg(self, **cfg):
         self._engine_cfg = cfg
@@ -157,6 +162,11 @@ class TFLocoformerSeparator(_SeparatorBase):
             input = input[:, 0]
         if not input.is_complex() or input.ndim != 3:
             raise ValueError("input must be a complex spectrogram [B, T, F] or [B, 1, T, F]")
+        if wants_autograd(self, list(self.parameters())):
+            _require_cuda(input, "input")
+            eng = self._ready()
+            ri = torch.view_as_real(input.detach().to(torch.complex64).contiguous())
+            return torch.view_as_complex(SeparatorFunction.apply(self, ri, *[self._param_refs[k] for k in eng.keys]))
         eng, prec = self._ready(), _resolve_precision(self)
         ri = torch.view_as_real(input.to(torch.complex64).contiguous())
         return torch.view_as_complex(eng.separator_forward(ri, prec))
@@ -250,31 +260,34 @@ class BSLocoformerSeparator(_SeparatorBase):
         fp = tuple((t.data_ptr(), t._version) for t in tensors)
         if self._bs_pack is not None and self._bs_pack[0] == fp:
             return self._bs_pack[1], self._bs_pack[2]
-        chunks, table, off = [], [], 0
+        chunks, table, off, where = [], [], 0, {}
 
-        def add(t):
+        def add(t, src=None):
             nonlocal off
             flat = t.detach().to(device=device, dtype=torch.float32).reshape(-1)
             chunks.append(flat)
             start = off
             off += flat.numel()
+            where[id(t if src is None else src)] = (start, src is not None)
             return start
 
         for b, width in enumerate(bsm.bands):
             sp, de = bsm.band_split_module[b], bsm.bandwise_decoding_module[b]
             row = [bsm.band_idx[b], width,
-                   add(sp[0].weight), add(sp[0].bias), add(sp[1].weight[:, :, 0].t().contiguous()), add(sp[1].bias),
-                   add(de[0].weight), add(de[0].bias), add(de[1].weight[:, :, 0].t().contiguous()), add(de[1].bias),
-                   add(de[3].weight[:, :, 0].t().contiguous()), add(de[3].bias),
-                   add(de[4].weight[:, :, 0].t().contiguous()), add(de[4].bias), 0, 0]
+                   add(sp[0].weight), add(sp[0].bias), add(sp[1].weight[:, :, 0].t().contiguous(), sp[1].weight),
+                   add(sp[1].bias), add(de[0].weight), add(de[0].bias),
+                   add(de[1].weight[:, :, 0].t().contiguous(), de[1].weight), add(de[1].bias),
+                   add(de[3].weight[:, :, 0].t().contiguous(), de[3].weight), add(de[3].bias),
+                   add(de[4].weight[:, :, 0].t().contiguous(), de[4].weight), add(de[4].bias), 0, 0]
             table.append(row)
         wbuf = torch.cat(chunks)
         tab = torch.tensor(table, dtype=torch.int64, device=device)
-        self._bs_pack = (fp, wbuf, tab)
+        # per parameter (bs_band_params order): (offset in wbuf, stored transposed) -- where its gradient lands
+        self._bs_pack = (fp, wbuf, tab, [where[id(t)] for t in tensors])
         return wbuf, tab
 
     def forward(self, input: torch.Tensor) -> torch.Tensor:
-        from .engine import _require_cuda, _stream
+        from .engine import _stream
         from ._lib import check
         _forward_only(self, input)
         if input.ndim == 3:
@@ -287,6 +300,12 @@ class BSLocoformerSeparator(_SeparatorBase):
         _require_cuda(spec, "input")
         B, M, T, F = spec.shape
         assert M == (2 if self.stereo else 1), (M, self.stereo)
+        if wants_autograd(self, list(self.parameters())):
+            eng = self._ready()
+            ri = torch.view_as_real(spec.detach().to(torch.complex64).contiguous())
+            params = [self._param_refs[k] for k in eng.keys] + bs_band_params(self)
+            out = torch.view_as_complex(BSFunction.apply(self, ri, *params))    # [B, S, M, T, F]
+            return out if self.stereo else out[:, :, 0]
         eng, prec = self._ready(), _resolve_precision(self)
         bsm = self.band_split_module
         nb, C, S = len(bsm.bands), self.emb_dim, self.num_spk
