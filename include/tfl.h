@@ -178,6 +178,21 @@ int tfl_sep_train_forward(const tfl_plan* plan, const void* packed, const float*
 int tfl_sep_train_backward(const tfl_plan* plan, const void* packed, const float* const* weights, int n_weights,
                            const float* d_est, const float* spec, int batch, int n_frames, int n_freq, float* grads,
                            void* workspace, size_t ws_bytes, tfl_stream_t stream);
+/* tfl_sep_train_backward plus the input gradient d_spec [B, Tf, F, 2] (overwritten). */
+int tfl_sep_train_backward_input(const tfl_plan* plan, const void* packed, const float* const* weights, int n_weights,
+                                 const float* d_est, const float* spec, int batch, int n_frames, int n_freq, float* grads,
+                                 void* workspace, size_t ws_bytes, tfl_stream_t stream, float* d_spec);
+/* TFLocoformerMSS (plan with the STFT and enc_in_ch == 2, at most 4 sources, n_samples > n_fft/2).  The workspace holds
+ * the saved forward, the spectrogram and the buffers of the mixture gradient; no loss buffers. */
+size_t tfl_mss_train_workspace_bytes(const tfl_plan* plan, int batch, int n_samples);
+/* mixture [B, T] -> audio [S, B, T] and / or est [B, S, Tf, F, 2] (either may be NULL). */
+int tfl_mss_train_forward(const tfl_plan* plan, const void* packed, const float* mixture, int batch, int n_samples,
+                          float* audio, float* est, void* workspace, size_t ws_bytes, tfl_stream_t stream);
+/* Exactly one of d_audio [S, B, T] / d_est [B, S, Tf, F, 2] -> grads (tfl_train_grad_layout, overwritten) and, when
+ * d_mixture is not NULL, d_mixture [B, T] (overwritten).  Same packed image and workspace as the forward. */
+int tfl_mss_train_backward(const tfl_plan* plan, const void* packed, const float* const* weights, int n_weights,
+                           const float* d_audio, const float* d_est, int batch, int n_samples, float* grads,
+                           float* d_mixture, void* workspace, size_t ws_bytes, tfl_stream_t stream);
 /* Blocks-only plan (enc_in_ch == 0): x_in [B, Tf, F, C] -> x_out (all Locoformer blocks); backward: dx_out -> dx_in and
  * grads (overwritten).  x_in / x_out and dx_out / dx_in may not overlap. */
 int tfl_blocks_train_forward(const tfl_plan* plan, const void* packed, const float* x_in, int batch, int n_frames,

@@ -63,6 +63,10 @@ SIGNATURES = {  # name -> (restype, argtypes); must list every symbol of include
     "tfl_sep_train_workspace_bytes": (_Z, [_P, _I, _I, _I]),
     "tfl_sep_train_forward": (_I, [_P, _P, _P, _I, _I, _I, _P, _P, _Z, _P]),
     "tfl_sep_train_backward": (_I, [_P, _P, C.POINTER(_P), _I, _P, _P, _I, _I, _I, _P, _P, _Z, _P]),
+    "tfl_sep_train_backward_input": (_I, [_P, _P, C.POINTER(_P), _I, _P, _P, _I, _I, _I, _P, _P, _Z, _P, _P]),
+    "tfl_mss_train_workspace_bytes": (_Z, [_P, _I, _I]),
+    "tfl_mss_train_forward": (_I, [_P, _P, _P, _I, _I, _P, _P, _P, _Z, _P]),
+    "tfl_mss_train_backward": (_I, [_P, _P, C.POINTER(_P), _I, _P, _P, _I, _I, _P, _P, _P, _Z, _P]),
     "tfl_blocks_train_forward": (_I, [_P, _P, _P, _I, _I, _I, _P, _P, _Z, _P]),
     "tfl_blocks_train_backward": (_I, [_P, _P, C.POINTER(_P), _I, _P, _I, _I, _I, _P, _P, _P, _Z, _P]),
     "tfl_grad_clip_norm":(_I, [_P, _L, _F, _P, _P, _Z, _P]),

@@ -1,17 +1,19 @@
-"""Training of the spectrogram separators through torch autograd (DESIGN.md section 8b).
+"""Training of the models through torch autograd (DESIGN.md section 8b).
 
-``TFLocoformerSeparator`` (and its ESPnet adapter) and ``BSLocoformerSeparator`` run their forward as a
-``torch.autograd.Function`` when the model is built or set with ``differentiable = True``, is in training mode, grad is
-enabled and some parameter requires grad.  The forward keeps its activations in a workspace of its own (one per call, so
-two forwards before one backward do not share saved state); the backward is CUDA (include/tfl.h:
-``tfl_sep_train_backward``, ``tfl_blocks_train_backward``, ``tfl_bs_band_decode_bwd``, ``tfl_bs_band_split_bwd``) and
-returns every parameter's gradient in the reference's tensor layout, so any torch loss, optimiser, gradient clipping or
-DDP wrapper drives the model as it would the reference.
+``TFLocoformerMSS``, ``TFLocoformerSeparator`` (and its ESPnet adapter) and ``BSLocoformerSeparator`` run their forward
+as a ``torch.autograd.Function`` when the model is built or set with ``differentiable = True``, is in training mode, grad
+is enabled and some parameter requires grad (for ``TFLocoformerMSS`` and ``TFLocoformerSeparator``: or the input does).
+The forward keeps its activations in a workspace of its own (one per call, so two forwards before one backward do not
+share saved state); the backward is CUDA (include/tfl.h: ``tfl_mss_train_backward``, ``tfl_sep_train_backward[_input]``,
+``tfl_blocks_train_backward``, ``tfl_bs_band_decode_bwd``, ``tfl_bs_band_split_bwd``) and returns every parameter's
+gradient in the reference's tensor layout, so any torch loss, optimiser, gradient clipping or DDP wrapper drives the
+model as it would the reference.
 
 Arithmetic follows ``TFL_OPT_TRAIN_MODE`` exactly as the MSS training step (``training.Trainer``) does: fp32, tf32, or
 (the default) mixed -- the sub-block forward on the bf16 tcgen05 kernels, encoder / decoder and backward on tf32.  The
-model's ``precision`` attribute selects the inference arithmetic only.  No gradient reaches the input spectrogram: an
-input that requires grad is refused, as on the inference path.
+model's ``precision`` attribute selects the inference arithmetic only.  ``TFLocoformerMSS`` returns a gradient for the
+mixture and ``TFLocoformerSeparator`` one for its complex input spectrogram; ``BSLocoformerSeparator`` refuses an input
+that requires grad, as the inference path does.
 """
 import ctypes as C
 from typing import List
@@ -23,10 +25,11 @@ from ._lib import check
 from .engine import _stream
 
 
-def wants_autograd(model, params: List[torch.Tensor]) -> bool:
-    """True when ``model``'s forward must build a graph: opted in, training mode, grad enabled, a parameter requires grad."""
+def wants_autograd(model, params: List[torch.Tensor], *inputs: torch.Tensor) -> bool:
+    """True when ``model``'s forward must build a graph: opted in, training mode, grad enabled, and a parameter or one of
+    ``inputs`` requires grad."""
     return (bool(getattr(model, "differentiable", False)) and model.training and torch.is_grad_enabled()
-            and any(p.requires_grad for p in params))
+            and any(t.requires_grad for t in list(params) + list(inputs)))
 
 
 def _grad_layout(eng):
@@ -57,13 +60,59 @@ def _raw(params):
     return out
 
 
-def _unflatten(eng, grads: torch.Tensor, params) -> List:
+def _unflatten(eng, grads: torch.Tensor, params, needs=None) -> List:
+    """Per-parameter views of the flat buffer; None where the tensor is not trainable or (``needs``) wants no gradient."""
     offs, sizes, _ = _grad_layout(eng)
-    return [None if o < 0 else grads[o:o + n].view(p.shape) for p, o, n in zip(params, offs, sizes)]
+    needs = [True] * len(params) if needs is None else needs
+    return [None if o < 0 or not w else grads[o:o + n].view(p.shape) for p, o, n, w in zip(params, offs, sizes, needs)]
+
+
+class MSSFunction(torch.autograd.Function):
+    """mixture [B, T] -> audio [S, B, T] (``want_audio``) or est [B, S, Tf, F, 2] of a TFLocoformerMSS; differentiable in
+    the parameters and the mixture."""
+
+    @staticmethod
+    def forward(ctx, model, mixture, want_audio, *params):
+        eng = model._engine
+        lib = eng.lib
+        B, T = mixture.shape
+        S, n_fft, hop = eng.cfg["n_src"], eng.cfg["n_fft"], eng.cfg["hop"]
+        dev = mixture.device
+        ws = torch.empty(max(256, lib.tfl_mss_train_workspace_bytes(eng.plan, B, T)), dtype=torch.uint8, device=dev)
+        shape = (S, B, T) if want_audio else (B, S, 1 + T // hop, n_fft // 2 + 1, 2)
+        out = torch.empty(shape, dtype=torch.float32, device=dev)
+        packed = eng.packed
+        with torch.cuda.device(dev):
+            check(lib.tfl_mss_train_forward(eng.plan, packed.data_ptr(), mixture.data_ptr(), B, T,
+                                            out.data_ptr() if want_audio else None,
+                                            None if want_audio else out.data_ptr(), ws.data_ptr(), ws.numel(),
+                                            _stream()))
+        ctx.eng, ctx.want_audio, ctx.shape = eng, want_audio, (B, T)
+        ctx.save_for_backward(packed, ws, *params)
+        return out
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, d_out):
+        eng = ctx.eng
+        packed, ws, *params = ctx.saved_tensors
+        raw = _raw(params)
+        B, T = ctx.shape
+        dev = ws.device
+        grads = torch.empty(_grad_layout(eng)[2], dtype=torch.float32, device=dev)
+        d_out = d_out.to(torch.float32).contiguous()
+        d_mix = torch.empty((B, T), dtype=torch.float32, device=dev) if ctx.needs_input_grad[1] else None
+        with torch.cuda.device(dev):
+            check(eng.lib.tfl_mss_train_backward(eng.plan, packed.data_ptr(), _weights_array(raw), len(raw),
+                                                 d_out.data_ptr() if ctx.want_audio else None,
+                                                 None if ctx.want_audio else d_out.data_ptr(), B, T, grads.data_ptr(),
+                                                 None if d_mix is None else d_mix.data_ptr(), ws.data_ptr(), ws.numel(),
+                                                 _stream()))
+        return (None, d_mix, None, *_unflatten(eng, grads, params, ctx.needs_input_grad[3:]))
 
 
 class SeparatorFunction(torch.autograd.Function):
-    """spec [B, Tf, F, 2] -> est [B, S, Tf, F, 2] of a TFLocoformerSeparator; differentiable in the parameters."""
+    """spec [B, Tf, F, 2] -> est [B, S, Tf, F, 2] of a TFLocoformerSeparator; differentiable in the parameters and spec."""
 
     @staticmethod
     def forward(ctx, model, spec_ri, *params):
@@ -90,11 +139,15 @@ class SeparatorFunction(torch.autograd.Function):
         B, Tf, F, _ = spec_ri.shape
         grads = torch.empty(_grad_layout(eng)[2], dtype=torch.float32, device=spec_ri.device)
         d_est = d_est.to(torch.float32).contiguous()
+        args = (eng.plan, packed.data_ptr(), _weights_array(raw), len(raw), d_est.data_ptr(), spec_ri.data_ptr(), B, Tf, F,
+                grads.data_ptr(), ws.data_ptr(), ws.numel(), _stream())
+        d_spec = torch.empty_like(spec_ri) if ctx.needs_input_grad[1] else None
         with torch.cuda.device(spec_ri.device):
-            check(eng.lib.tfl_sep_train_backward(eng.plan, packed.data_ptr(), _weights_array(raw), len(raw),
-                                                 d_est.data_ptr(), spec_ri.data_ptr(), B, Tf, F, grads.data_ptr(),
-                                                 ws.data_ptr(), ws.numel(), _stream()))
-        return (None, None, *_unflatten(eng, grads, params))
+            if d_spec is None:
+                check(eng.lib.tfl_sep_train_backward(*args))
+            else:
+                check(eng.lib.tfl_sep_train_backward_input(*args, d_spec.data_ptr()))
+        return (None, d_spec, *_unflatten(eng, grads, params, ctx.needs_input_grad[2:]))
 
 
 def bs_band_params(model) -> List[torch.Tensor]:

@@ -579,6 +579,102 @@ __global__ void __launch_bounds__(256) enc_wgrad_kernel(const float* __restrict_
   }
 }
 
+// pass 3 (input gradient, only when the caller wants d spec): dv as in pass 2, then the transposed 3x3 conv
+//   dspec[t', f', i] = sum_{dt, df, c} dv[t' - dt + 1, f' - df + 1, c] * w[(dt*3+df)*CIN + i][c]   (zero outside the image)
+// split as P[pos][j] = sum_c dv[pos][c] w[j][c] (j = (dt*3+df)*CIN + i; one warp per position, lanes over channels) and a
+// 9-tap gather of P.  A CTA owns ENC_IG_TT frames x ENC_IG_FT bins; P of the tile plus a one-position halo lives in shared
+// memory, so each v / dy row is read once per CTA that needs it (interior rows once, halo rows by two or four CTAs).
+constexpr int ENC_IG_TT = 8, ENC_IG_FT = 32;
+template <int CIN>
+__global__ void __launch_bounds__(256) enc_input_grad_kernel(const float* __restrict__ v, const float* __restrict__ dy,
+                                                             int n_frames, int n_freq, int C, const float* __restrict__ stats,
+                                                             const double* __restrict__ sums, const float* __restrict__ gw,
+                                                             const float* __restrict__ w /*[9][CIN][C]*/,
+                                                             float* __restrict__ dspec /*[B][Tf][F][CIN]*/) {
+  constexpr int J = 9 * CIN;
+  static_assert(J <= 32, "one lane per tap-channel pair");
+  constexpr int HT = ENC_IG_TT + 2, HF = ENC_IG_FT + 2;
+  extern __shared__ float ig_sm[];            // wsm [J][C], then P [HT * HF][J]
+  float* wsm = ig_sm;
+  float* P = ig_sm + (size_t)J * C;
+  const int b = blockIdx.z, t0 = blockIdx.y * ENC_IG_TT, f0 = blockIdx.x * ENC_IG_FT;
+  for (int i = threadIdx.x; i < J * C; i += blockDim.x) wsm[i] = w[i];
+  __syncthreads();
+  const long long per_sample_pos = (long long)n_frames * n_freq;
+  const float mean = stats[b * 2], rstd = stats[b * 2 + 1];
+  const double cnt = (double)per_sample_pos * C;
+  const float m1 = (float)(sums[b * 2] / cnt), m2 = (float)(sums[b * 2 + 1] / cnt);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, n_warps = blockDim.x >> 5;
+  for (int hp = warp; hp < HT * HF; hp += n_warps) {
+    const int t = t0 - 1 + hp / HF, f = f0 - 1 + hp % HF;
+    float a[32];
+#pragma unroll
+    for (int j = 0; j < 32; ++j) a[j] = 0.f;
+    if (t >= 0 && t < n_frames && f >= 0 && f < n_freq) {
+      const size_t row = ((size_t)b * per_sample_pos + (size_t)t * n_freq + f) * C;
+      for (int c = lane; c < C; c += 32) {
+        const float vh = (__ldg(&v[row + c]) - mean) * rstd;
+        const float dv = rstd * (__ldg(&dy[row + c]) * __ldg(&gw[c]) - m1 - vh * m2);
+#pragma unroll
+        for (int j = 0; j < J; ++j) a[j] = fmaf(dv, wsm[j * C + c], a[j]);
+      }
+    }
+    // transpose-reduce over the warp: after the step of width s, a lane keeps the half of its s-wide window selected by
+    // its lane bit s; at the end lane l holds the warp total of value l
+#pragma unroll
+    for (int s = 16; s >= 1; s >>= 1) {
+      const bool upper = (lane & s) != 0;
+#pragma unroll
+      for (int j = 0; j < s; ++j) {
+        const float send = upper ? a[j] : a[j + s];
+        const float keep = upper ? a[j + s] : a[j];
+        a[j] = keep + __shfl_xor_sync(0xffffffffu, send, s);
+      }
+    }
+    if (lane < J) P[hp * J + lane] = a[0];
+  }
+  __syncthreads();
+  for (int o = threadIdx.x; o < ENC_IG_TT * ENC_IG_FT * CIN; o += blockDim.x) {
+    const int i = o % CIN, q = o / CIN, lt = q / ENC_IG_FT, lf = q % ENC_IG_FT;
+    const int t = t0 + lt, f = f0 + lf;
+    if (t >= n_frames || f >= n_freq) continue;
+    float acc = 0.f;
+#pragma unroll
+    for (int dt = 0; dt < 3; ++dt)
+#pragma unroll
+      for (int df = 0; df < 3; ++df)       // source position (t - dt + 1, f - df + 1) = halo cell (lt - dt + 2, lf - df + 2)
+        acc += P[((lt - dt + 2) * HF + (lf - df + 2)) * J + (dt * 3 + df) * CIN + i];
+    dspec[(((size_t)b * n_frames + t) * n_freq + f) * CIN + i] = acc;
+  }
+}
+
+// ---- adjoint of reflect pad -> frame: dmix[b][n] = sum of the windowed frame adjoints (stft_adj_frames_kernel output)
+// over every frame that covers padded coordinate n + pad, plus the reflected images pad - n (1 <= n <= pad) and
+// pad + 2 (T - 1) - n (right pad).  The same fold as in loss_grad_kernel, for the model's own STFT.
+__global__ void __launch_bounds__(256) stft_fold_kernel(const float* __restrict__ frames /*[b][t][n_fft]*/, int n_samples,
+                                                        int n_fft, int hop, int n_frames, float* __restrict__ dmix /*[b][n]*/) {
+  const int b = blockIdx.y, pad = n_fft >> 1;
+  const float* fr = frames + (size_t)b * n_frames * n_fft;
+  auto gather = [&](long long p) -> float {
+    long long t_hi = p / hop;
+    if (t_hi > n_frames - 1) t_hi = n_frames - 1;
+    const long long t_lo = p - n_fft + 1 <= 0 ? 0 : (p - n_fft + hop) / hop;
+    float acc = 0.f;
+    for (long long tp = t_lo; tp <= t_hi; ++tp) acc += __ldg(&fr[tp * n_fft + (p - tp * hop)]);
+    return acc;
+  };
+  const long long covered = (long long)(n_frames - 1) * hop + n_fft;
+  for (long long n = (long long)blockIdx.x * blockDim.x + threadIdx.x; n < n_samples; n += (long long)gridDim.x * blockDim.x) {
+    float g = gather(n + pad);
+    if (n >= 1 && n <= pad) g += gather(pad - n);
+    if (n <= n_samples - 2) {
+      const long long p = pad + 2 * ((long long)n_samples - 1) - n;
+      if (p < covered) g += gather(p);
+    }
+    dmix[(size_t)b * n_samples + n] = g;
+  }
+}
+
 // ---- iSTFT backward: dEst[b][src][t][k] = (c_k / N) * rfft(w .* u[t * hop : t * hop + N])_k, u = dAudio / envelope on the
 // valid samples and zero elsewhere (c_0 = c_{N/2} = 1, else 2; imaginary parts of DC / Nyquist get no gradient: :56-75) ----
 __global__ void __launch_bounds__(256) istft_bwd_kernel(const float* __restrict__ daudio /*[src][b][n]*/, int n_src, int batch,

@@ -56,6 +56,7 @@ struct TrainWs {
   size_t fwd16_base;
   size_t ckpt, dx, dxn, scratch, lse, dbuf, nat, wt, dest, audio, daudio;
   size_t s5, stats_scratch, coef, loss_rows, l1_rows, spec_rows, ltab_tw, ltab_win, lspec_e, lspec_t, lframes, enc_sums;
+  size_t dspec, adj_frames;  // saved mode with T > 0 (the MSS autograd pair): d spec [B][Tf][F][2], frame adjoints [B][Tf][n_fft]
   size_t total;
   // inside `scratch` (FFN and attention backward never overlap in time)
   size_t dg, hid2, dh;       // FFN: dG, recomputed hidden, dH
@@ -64,7 +65,8 @@ struct TrainWs {
 };
 
 // (B, Tf, F) size the network buffers; T (audio samples, 0 = stage-level use) and the loss STFT size the rest.
-// `saved` (frames-only mode, T = 0): the checkpoint slots of one saved forward without the STFT / loss buffers.
+// `saved`: the checkpoint slots of one saved forward, without the loss buffers.  T = 0: the separators' frames-only
+// mode; T > 0: TFLocoformerMSS, plus the buffers of the mixture gradient (d spec and the adjoint STFT frames).
 static TrainWs plan_train_ws(const tfl_plan* pl, int B, int Tf, int F, int T, int l_fft, int l_hop, bool saved = false) {
   const tfl_config& c = pl->cfg;
   TrainWs w{};
@@ -100,15 +102,20 @@ static TrainWs plan_train_ws(const tfl_plan* pl, int B, int Tf, int F, int T, in
   // transposed weights of the data-gradient GEMMs of one FFN: [K][C][H] and [K][2H][C]
   w.wt = take((K * C * Hmax + K * 2 * Hmax * C) * sizeof(float));
   w.dest = take(N * 2 * S * sizeof(float));
-  w.audio = take(S * B * (size_t)T * sizeof(float));
-  w.daudio = take(S * B * (size_t)T * sizeof(float));
   const size_t rows = S * B;
-  w.s5 = take(rows * 5 * sizeof(double));
-  w.stats_scratch = take(rows * STATS_BLOCKS * 5 * sizeof(double));
-  w.coef = take(rows * 3 * sizeof(float));
-  w.loss_rows = take(rows * sizeof(double));
-  w.l1_rows = take(rows * sizeof(double));
-  w.spec_rows = take(rows * sizeof(double));
+  if (!saved) {
+    w.audio = take(S * B * (size_t)T * sizeof(float));
+    w.daudio = take(S * B * (size_t)T * sizeof(float));
+    w.s5 = take(rows * 5 * sizeof(double));
+    w.stats_scratch = take(rows * STATS_BLOCKS * 5 * sizeof(double));
+    w.coef = take(rows * 3 * sizeof(float));
+    w.loss_rows = take(rows * sizeof(double));
+    w.l1_rows = take(rows * sizeof(double));
+    w.spec_rows = take(rows * sizeof(double));
+  } else if (T > 0) {
+    w.dspec = take(N * 2 * sizeof(float));
+    w.adj_frames = take((size_t)B * Tf * c.n_fft * sizeof(float));
+  }
   w.enc_sums = take((size_t)B * 2 * sizeof(double));
   w.l_frames = (l_fft > 0 && T > 0) ? 1 + T / l_hop : 0;
   w.l_freq = l_fft / 2 + 1;
@@ -438,9 +445,9 @@ static int dec_backward(const tfl_plan* pl, const char* pk, const GradLayout& gl
 }
 
 // Encoder backward from tw.dx = dL/d(encoder output): v = conv(spec) recomputed into xn, then GroupNorm(1, C) backward
-// and the conv weight gradient.  No gradient for spec.
+// and the conv weight gradient; with d_spec, also dL/d spec [B, Tf, F, 2] (overwritten).
 static int enc_backward(const tfl_plan* pl, const char* pk, const GradLayout& gl, float* grads, const float* spec, Dims d,
-                        const TrainWs& tw, char* wsp, cudaStream_t st) {
+                        const TrainWs& tw, char* wsp, cudaStream_t st, float* d_spec = nullptr) {
   const tfl_config& c = pl->cfg;
   const int C = c.emb_dim, B = d.B, Tf = d.Tf, F = d.F;
   const int cthreads = (C + 31) / 32 * 32;
@@ -468,11 +475,20 @@ static int enc_backward(const tfl_plan* pl, const char* pk, const GradLayout& gl
   permute(nat, grads + gl.off[0], 1, C, 2, 9, 0, 1, C, (long long)2 * C, 0, -1, st);
   permute(nat + (size_t)18 * C, grads + gl.off[1], 1, 1, 1, C, 0, 0, 0, 1, 0, -1, st);
   TFL_LAUNCH_CHECK();
+  if (d_spec != nullptr) {
+    const size_t ism = ((size_t)18 * C + (size_t)(ENC_IG_TT + 2) * (ENC_IG_FT + 2) * 18) * sizeof(float);
+    TFL_CUDA(opt_in_smem(enc_input_grad_kernel<2>, ism));
+    const dim3 grid((F + ENC_IG_FT - 1) / ENC_IG_FT, (Tf + ENC_IG_TT - 1) / ENC_IG_TT, B);
+    enc_input_grad_kernel<2><<<grid, 256, ism, st>>>(v, dx, Tf, F, C, stats, sums, (const float*)(pk + pl->lay.gln_w),
+                                                     (const float*)(pk + pl->lay.enc_w), d_spec);
+    TFL_LAUNCH_CHECK();
+  }
   return 0;
 }
 
 // Shared argument checks of the saved-forward / backward pairs; fills the workspace plan.
-static int check_saved(const tfl_plan* pl, const void* packed, int B, int Tf, int F, bool conv, size_t ws_bytes, TrainWs* tw) {
+static int check_saved(const tfl_plan* pl, const void* packed, int B, int Tf, int F, bool conv, size_t ws_bytes, TrainWs* tw,
+                       int T = 0) {
   TFL_CHECK(pl && packed, "null argument");
   TFL_CHECK(B >= 1 && Tf >= 1 && F >= 1, "empty input (batch %d, frames %d, bins %d)", B, Tf, F);
   TFL_CHECK(pl->cfg.emb_dim <= 256, "training kernels support emb_dim <= 256");
@@ -482,10 +498,40 @@ static int check_saved(const tfl_plan* pl, const void* packed, int B, int Tf, in
   } else {
     TFL_CHECK(pl->cfg.enc_in_ch == 0, "this entry point needs a blocks-only plan (enc_in_ch == 0)");
   }
-  *tw = plan_train_ws(pl, B, Tf, F, 0, 0, 0, /*saved=*/true);
+  *tw = plan_train_ws(pl, B, Tf, F, T, 0, 0, /*saved=*/true);
   TFL_CHECK(ws_bytes >= tw->total, "workspace too small (%zu < %zu)", ws_bytes, tw->total);
   if (ensure_device_ready()) return -1;
   return timeout_pending();
+}
+
+// The TFLocoformerMSS pair: plan with STFT and conv encoder, T past the reflect padding; (Tf, F) from T.
+static int check_mss(const tfl_plan* pl, const void* packed, int B, int T, size_t ws_bytes, TrainWs* tw, Dims* d) {
+  TFL_CHECK(pl && packed, "null argument");
+  const tfl_config& c = pl->cfg;
+  TFL_CHECK(c.n_fft > 0 && c.enc_in_ch == 2, "this entry point needs the full TFLocoformerMSS plan (STFT + conv encoder)");
+  TFL_CHECK(B >= 1 && T > c.n_fft / 2, "reflect padding needs more than n_fft/2 = %d samples (got %d)", c.n_fft / 2, T);
+  *d = Dims{B, 1 + T / c.hop, c.n_fft / 2 + 1};
+  return check_saved(pl, packed, B, d->Tf, d->F, true, ws_bytes, tw, T);
+}
+
+// tfl_sep_train_backward, with dL/d spec into d_spec when it is not NULL.
+static int sep_backward(const tfl_plan* pl, const void* packed, const float* const* w, int n_weights, const float* d_est,
+                        const float* spec, int B, int Tf, int F, float* grads, void* workspace, size_t ws_bytes,
+                        float* d_spec, cudaStream_t st) {
+  Tf32Scope tf32_scope;
+  if (check_train(pl, packed, w, n_weights)) return -1;
+  TrainWs tw;
+  if (check_saved(pl, packed, B, Tf, F, true, ws_bytes, &tw)) return -1;
+  TFL_CHECK(d_est && spec && grads && workspace, "null argument");
+  const Dims d{B, Tf, F};
+  const char* pk = (const char*)packed;
+  char* wsp = (char*)workspace;
+  const GradLayout gl = grad_layout(pl);
+  TFL_CUDA(cudaMemsetAsync(grads, 0, (size_t)gl.total * sizeof(float), st));
+  const float* x = ckpt_slot(tw, wsp, d, pl->cfg.emb_dim, (size_t)tw.n_sub);
+  if (dec_backward(pl, pk, gl, grads, n_weights, x, d_est, d, tw, wsp, st)) return -1;
+  if (blocks_backward(pl, pk, w, gl, grads, d, tw, wsp, st)) return -1;
+  return enc_backward(pl, pk, gl, grads, spec, d, tw, wsp, st, d_spec);
 }
 
 }  // namespace tfl
@@ -687,21 +733,95 @@ int tfl_sep_train_backward(const tfl_plan* pl, const void* packed, const float* 
                            const float* spec, int B, int Tf, int F, float* grads, void* workspace, size_t ws_bytes,
                            tfl_stream_t stream) {
   NvtxRange nvtx_range("tfl::sep_train_backward");
+  return sep_backward(pl, packed, w, n_weights, d_est, spec, B, Tf, F, grads, workspace, ws_bytes, nullptr,
+                      (cudaStream_t)stream);
+}
+
+// tfl_sep_train_backward plus the input gradient d_spec [B, Tf, F, 2] (overwritten).
+int tfl_sep_train_backward_input(const tfl_plan* pl, const void* packed, const float* const* w, int n_weights,
+                                 const float* d_est, const float* spec, int B, int Tf, int F, float* grads, void* workspace,
+                                 size_t ws_bytes, tfl_stream_t stream, float* d_spec) {
+  NvtxRange nvtx_range("tfl::sep_train_backward_input");
+  TFL_CHECK(d_spec, "null argument");
+  return sep_backward(pl, packed, w, n_weights, d_est, spec, B, Tf, F, grads, workspace, ws_bytes, d_spec,
+                      (cudaStream_t)stream);
+}
+
+size_t tfl_mss_train_workspace_bytes(const tfl_plan* pl, int B, int T) {
+  if (pl == nullptr || pl->cfg.n_fft <= 0 || B < 1 || T < 1) return 0;
+  return plan_train_ws(pl, B, 1 + T / pl->cfg.hop, pl->cfg.n_fft / 2 + 1, T, 0, 0, /*saved=*/true).total;
+}
+
+// TFLocoformerMSS forward with the sub-block inputs and the spectrogram saved in `workspace` for tfl_mss_train_backward:
+// the forward of tfl_train_forward_backward (STFT, encoder, saved blocks, decoder, iSTFT) without the loss.
+int tfl_mss_train_forward(const tfl_plan* pl, const void* packed, const float* mixture, int B, int T, float* audio,
+                          float* est, void* workspace, size_t ws_bytes, tfl_stream_t stream) {
+  NvtxRange nvtx_range("tfl::mss_train_forward");
+  Tf32Scope tf32_scope;
+  TrainWs tw;
+  Dims d;
+  if (check_mss(pl, packed, B, T, ws_bytes, &tw, &d)) return -1;
+  TFL_CHECK(mixture && workspace, "null argument");
+  const int C = pl->cfg.emb_dim;
+  const bool mixed = tfl_option(TFL_OPT_TRAIN_MODE) >= 2;
+  const int prec = mixed ? TFL_PRECISION_BF16 : TFL_PRECISION_FP32;
+  char* wsp = (char*)workspace;
+  cudaStream_t st = (cudaStream_t)stream;
+  float* spec = (float*)(wsp + tw.fwd.spec);
+  float* e = est != nullptr ? est : (float*)(wsp + tw.fwd.est);
+  if (tfl_stft(pl, packed, mixture, B, T, spec, stream)) return -1;
+  if (enc_conv_gln_any(pl, packed, spec, B, d.Tf, d.F, ckpt_slot(tw, wsp, d, C, 0), workspace, ws_bytes, prec, stream)) return -1;
+  if (saved_blocks_forward(pl, (const char*)packed, d, tw, wsp, mixed, st)) return -1;
+  if (dec_conv_any(pl, packed, ckpt_slot(tw, wsp, d, C, (size_t)tw.n_sub), B, d.Tf, d.F, e, prec, stream)) return -1;
+  if (audio != nullptr) return tfl_istft_ola(pl, packed, e, B, d.Tf, T, audio, stream);
+  return 0;
+}
+
+// Backward of tfl_mss_train_forward from d_audio [S][B][T] or d_est [B][S][Tf][F][2] (exactly one): every parameter
+// gradient into `grads` (tfl_train_grad_layout, overwritten) and, when d_mixture is not NULL, dL/d mixture [B][T].
+int tfl_mss_train_backward(const tfl_plan* pl, const void* packed, const float* const* w, int n_weights, const float* d_audio,
+                           const float* d_est, int B, int T, float* grads, float* d_mixture, void* workspace,
+                           size_t ws_bytes, tfl_stream_t stream) {
+  NvtxRange nvtx_range("tfl::mss_train_backward");
   Tf32Scope tf32_scope;
   if (check_train(pl, packed, w, n_weights)) return -1;
   TrainWs tw;
-  if (check_saved(pl, packed, B, Tf, F, true, ws_bytes, &tw)) return -1;
-  TFL_CHECK(d_est && spec && grads && workspace, "null argument");
-  const Dims d{B, Tf, F};
+  Dims d;
+  if (check_mss(pl, packed, B, T, ws_bytes, &tw, &d)) return -1;
+  TFL_CHECK((d_audio == nullptr) != (d_est == nullptr), "exactly one of d_audio / d_est must be given");
+  TFL_CHECK(grads && workspace, "null argument");
+  const tfl_config& c = pl->cfg;
   const char* pk = (const char*)packed;
   char* wsp = (char*)workspace;
   cudaStream_t st = (cudaStream_t)stream;
   const GradLayout gl = grad_layout(pl);
+  const float2* twid = (const float2*)(pk + pl->lay.twiddle);
+  const float* win = (const float*)(pk + pl->lay.window);
+  const size_t fsm = (size_t)c.n_fft * sizeof(float2);
   TFL_CUDA(cudaMemsetAsync(grads, 0, (size_t)gl.total * sizeof(float), st));
-  const float* x = ckpt_slot(tw, wsp, d, pl->cfg.emb_dim, (size_t)tw.n_sub);
-  if (dec_backward(pl, pk, gl, grads, n_weights, x, d_est, d, tw, wsp, st)) return -1;
+  const float* dest = d_est;
+  if (d_audio != nullptr) {
+    TFL_CUDA(opt_in_smem(istft_bwd_kernel, fsm));
+    istft_bwd_kernel<<<dim3(d.Tf, c.n_src, B), 256, fsm, st>>>(d_audio, c.n_src, B, T, c.n_fft, ilog2(c.n_fft), c.hop, d.Tf,
+                                                               twid, win, (float*)(wsp + tw.dest));
+    TFL_LAUNCH_CHECK();
+    dest = (const float*)(wsp + tw.dest);
+  }
+  const float* x = ckpt_slot(tw, wsp, d, c.emb_dim, (size_t)tw.n_sub);
+  if (dec_backward(pl, pk, gl, grads, n_weights, x, dest, d, tw, wsp, st)) return -1;
   if (blocks_backward(pl, pk, w, gl, grads, d, tw, wsp, st)) return -1;
-  return enc_backward(pl, pk, gl, grads, spec, d, tw, wsp, st);
+  float* dspec = d_mixture != nullptr ? (float*)(wsp + tw.dspec) : nullptr;
+  if (enc_backward(pl, pk, gl, grads, (const float*)(wsp + tw.fwd.spec), d, tw, wsp, st, dspec)) return -1;
+  if (d_mixture == nullptr) return 0;
+  float* frames = (float*)(wsp + tw.adj_frames);
+  TFL_CUDA(opt_in_smem(stft_adj_frames_kernel, fsm));
+  stft_adj_frames_kernel<<<dim3(d.Tf, B), 256, fsm, st>>>((const float2*)dspec, c.n_fft, ilog2(c.n_fft), d.Tf, twid, win, frames);
+  TFL_LAUNCH_CHECK();
+  long long blocks = ((long long)T + 255) / 256;
+  if (blocks > (long long)pl->sm_count * 4) blocks = (long long)pl->sm_count * 4;
+  stft_fold_kernel<<<dim3((unsigned)blocks, B), 256, 0, st>>>(frames, T, c.n_fft, c.hop, d.Tf, d_mixture);
+  TFL_LAUNCH_CHECK();
+  return 0;
 }
 
 // The same pair for a blocks-only plan (enc_in_ch == 0): x_in [B, Tf, F, C] -> x_out, and from dL/dx_out the block

@@ -120,16 +120,22 @@ class Engine:
         return ws
 
     # ---- whole-model calls ---------------------------------------------------------
-    def mss_forward(self, mixture: torch.Tensor, precision: int, want_audio: bool, want_spec: bool):
-        """mixture [B, T] fp32 CUDA -> (audio [S, B, T] or None, est_spec [B, S, Tf, F, 2] or None)."""
+    def check_mixture(self, mixture: torch.Tensor):
+        """The mixture checks of TFLocoformerMSS.forward: a [B, T] CUDA tensor longer than the reflect padding."""
         _require_cuda(mixture, "mixture")
         if mixture.ndim != 2:
             raise ValueError(f"mixture must be [B, T], got {tuple(mixture.shape)}")
         B, T = mixture.shape
-        n_fft, hop, S = self.cfg["n_fft"], self.cfg["hop"], self.cfg["n_src"]
+        n_fft = self.cfg["n_fft"]
         if T <= n_fft // 2:  # same failure mode as torch.stft's reflect pad in the reference
             raise RuntimeError(f"Argument #4: Padding size should be less than the corresponding input dimension, "
                                f"but got: padding ({n_fft // 2}, {n_fft // 2}) at dimension 2 of input {[1, B, T]}")
+
+    def mss_forward(self, mixture: torch.Tensor, precision: int, want_audio: bool, want_spec: bool):
+        """mixture [B, T] fp32 CUDA -> (audio [S, B, T] or None, est_spec [B, S, Tf, F, 2] or None)."""
+        self.check_mixture(mixture)
+        B, T = mixture.shape
+        n_fft, hop, S = self.cfg["n_fft"], self.cfg["hop"], self.cfg["n_src"]
         x = mixture.detach().to(torch.float32).contiguous()
         Tf, F = 1 + T // hop, n_fft // 2 + 1
         dev = x.device

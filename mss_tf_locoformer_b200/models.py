@@ -6,18 +6,18 @@ import torch
 import torch.nn as nn
 
 from .engine import Engine
-from .autograd import BSFunction, SeparatorFunction, bs_band_params, wants_autograd
+from .autograd import BSFunction, MSSFunction, SeparatorFunction, bs_band_params, wants_autograd
 from .engine import _require_cuda
 from .modules import (MSSTransform, RotaryEmbedding, TFLocoformerBlock, SOURCE_NAMES, _forward_only,
-                      _resolve_precision)
+                      _no_training_dropout, _resolve_precision)
 
 
 class _SeparatorBase(nn.Module):
     """Shared plumbing: engine creation, lazy weight packing, sub-module call sites."""
 
     precision: Optional[str] = None  # None = follow torch.autocast (bf16) else fp32; or "fp32" / "bf16"
-    # True: in training mode with grad enabled, forward builds an autograd graph over the parameters (autograd.py;
-    # TFLocoformerSeparator and BSLocoformerSeparator).  TFLocoformerMSS trains through training.Trainer instead.
+    # True: in training mode with grad enabled, forward builds an autograd graph over the parameters and, for
+    # TFLocoformerMSS and TFLocoformerSeparator, the input (autograd.py).  training.Trainer does not need it.
     differentiable: bool = False
 
     def _init_engine_cfg(self, **cfg):
@@ -113,9 +113,18 @@ class TFLocoformerMSS(_SeparatorBase):
         self._attach_sites()
 
     def forward(self, mixture: torch.Tensor, return_time_domain: bool = True) -> Dict[str, torch.Tensor]:
-        _forward_only(self, mixture)
-        eng, prec = self._ready(), _resolve_precision(self)
-        audio, spec = eng.mss_forward(mixture, prec, want_audio=return_time_domain, want_spec=not return_time_domain)
+        _no_training_dropout(self)
+        if wants_autograd(self, list(self.parameters()), mixture):
+            _require_cuda(mixture, "mixture")
+            eng = self._ready()
+            eng.check_mixture(mixture)
+            out = MSSFunction.apply(self, mixture.to(torch.float32).contiguous(), return_time_domain,
+                                    *[self._param_refs[k] for k in eng.keys])
+            audio, spec = (out, None) if return_time_domain else (None, out)
+        else:
+            _forward_only(self, mixture)
+            eng, prec = self._ready(), _resolve_precision(self)
+            audio, spec = eng.mss_forward(mixture, prec, want_audio=return_time_domain, want_spec=not return_time_domain)
         if return_time_domain:
             return {name: audio[i] for i, name in enumerate(SOURCE_NAMES[: self.n_sources])}
         est = torch.view_as_complex(spec)  # [B, S, Tf, F]
@@ -156,16 +165,20 @@ class TFLocoformerSeparator(_SeparatorBase):
         self._attach_sites()
 
     def forward(self, input: torch.Tensor) -> torch.Tensor:
-        _forward_only(self, input)
+        _no_training_dropout(self)
+        grad = wants_autograd(self, list(self.parameters()), input)
+        if not grad:
+            _forward_only(self, input)
         if input.ndim == 4:
             assert input.shape[1] == 1, "Only monaural input is supported."
             input = input[:, 0]
         if not input.is_complex() or input.ndim != 3:
             raise ValueError("input must be a complex spectrogram [B, T, F] or [B, 1, T, F]")
-        if wants_autograd(self, list(self.parameters())):
+        if grad:
             _require_cuda(input, "input")
             eng = self._ready()
-            ri = torch.view_as_real(input.detach().to(torch.complex64).contiguous())
+            # not detached: autograd carries d spec back through view_as_real (torch's complex-gradient convention)
+            ri = torch.view_as_real(input.to(torch.complex64).contiguous())
             return torch.view_as_complex(SeparatorFunction.apply(self, ri, *[self._param_refs[k] for k in eng.keys]))
         eng, prec = self._ready(), _resolve_precision(self)
         ri = torch.view_as_real(input.to(torch.complex64).contiguous())

@@ -30,11 +30,15 @@ def _resolve_precision(owner) -> int:
     return PRECISIONS[p]
 
 
-def _forward_only(module: nn.Module, *tensors):
+def _no_training_dropout(module: nn.Module):
     if module.training and getattr(module, "_dropout_p", 0.0) > 0.0:
         raise NotImplementedError(
             "training-mode dropout is not implemented by the B200 forward path; call .eval() "
             "(parity with the reference is defined for eval mode only)")
+
+
+def _forward_only(module: nn.Module, *tensors):
+    _no_training_dropout(module)
     if torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in tensors):
         raise NotImplementedError("mss_tf_locoformer_b200 is forward-only (no autograd); run under torch.no_grad() "
                                   "with inputs that do not require grad")
