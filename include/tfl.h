@@ -261,9 +261,17 @@ int tfl_bs_band_split_bwd(const float* spec, const float* dx, int batch, int n_c
  *   TFL_OPT_DEC_KERNEL   bf16-mode decoder: 1 = dec_conv_mma_kernel (9-tap gather), 2 = dec_conv_scatter_kernel (every
  *                        input row read once, rolling output-frame accumulators in shared memory; default for
  *                        emb_dim in {32, 64, 96, 128})
- *   TFL_OPT_TRACE_BASE   first chunk / tile index the pipeline trace records (64 entries per event; default 0) */
+ *   TFL_OPT_TRACE_BASE   first chunk / tile index the pipeline trace records (64 entries per event; default 0)
+ *   TFL_OPT_DETERMINISTIC  1 = bitwise-reproducible training entry points: every reduction over rows of the backward pass
+ *                        (weight-gradient GEMM splits, bias / gamma / decoder / encoder gradients, encoder statistics, loss
+ *                        row sums) stores per-split or per-block partials that one kernel adds in index order, with grids
+ *                        sized from the shapes alone (never the SM count), instead of fp32 / double atomics.  0 (default) =
+ *                        atomics.  Read when a training call is made: the *_train_workspace_bytes queries add the partials
+ *                        buffer only when it is 1, so the option must have the same value for the size query, a saved
+ *                        forward and its backward.  The inference entry points are deterministic and ignore it.  The
+ *                        Python layer sets it from torch.are_deterministic_algorithms_enabled(). */
 enum { TFL_OPT_ATTN_KERNEL = 0, TFL_OPT_FFN_KERNEL = 1, TFL_OPT_TRACE_BASE = 2, TFL_OPT_TAIL_KERNEL = 3, TFL_OPT_PDL = 4,
-       TFL_OPT_TRAIN_MODE = 5, TFL_OPT_DEC_KERNEL = 6, TFL_OPT_COUNT = 8 };
+       TFL_OPT_TRAIN_MODE = 5, TFL_OPT_DEC_KERNEL = 6, TFL_OPT_DETERMINISTIC = 7, TFL_OPT_COUNT = 8 };
 int tfl_debug_set_option(int key, int value);
 
 /* Diagnostic: install (or clear with NULL) a device buffer of >= 16 * 64 uint64 in which block 0 of the tcgen05 FFN

@@ -1,4 +1,5 @@
 """ctypes binding of include/tfl.h.  There is NO fallback: a missing library is an error."""
+import contextlib
 import ctypes as C
 import os
 
@@ -102,3 +103,19 @@ def load():
 def check(status: int):
     if status != 0:
         raise TflError(load().tfl_last_error().decode(errors="replace") or f"tfl error {status}")
+
+
+OPT_DETERMINISTIC = 7   # include/tfl.h TFL_OPT_DETERMINISTIC
+
+
+@contextlib.contextmanager
+def deterministic_option(on: bool):
+    """TFL_OPT_DETERMINISTIC = ``on`` for the duration of one training call, then back to the default 0.  The training
+    entry points read it when called, and a workspace query, the saved forward sized by it and that forward's backward
+    must all see the same value: callers pass ``torch.are_deterministic_algorithms_enabled()`` as read at the forward."""
+    lib = load()
+    check(lib.tfl_debug_set_option(OPT_DETERMINISTIC, 1 if on else 0))
+    try:
+        yield
+    finally:
+        lib.tfl_debug_set_option(OPT_DETERMINISTIC, 0)

@@ -14,6 +14,10 @@ Arithmetic follows ``TFL_OPT_TRAIN_MODE`` exactly as the MSS training step (``tr
 model's ``precision`` attribute selects the inference arithmetic only.  ``TFLocoformerMSS`` returns a gradient for the
 mixture and ``TFLocoformerSeparator`` one for its complex input spectrogram; ``BSLocoformerSeparator`` refuses an input
 that requires grad, as the inference path does.
+
+Under ``torch.use_deterministic_algorithms(True)``, as read at the forward and recorded for its backward, every
+reduction of the backward pass runs in a fixed order (``TFL_OPT_DETERMINISTIC``): two identical forward + backward
+passes return bitwise-identical gradients.
 """
 import ctypes as C
 from typing import List
@@ -21,7 +25,7 @@ from typing import List
 import torch
 from torch.autograd.function import once_differentiable
 
-from ._lib import check
+from ._lib import check, deterministic_option
 from .engine import _stream
 
 
@@ -78,16 +82,17 @@ class MSSFunction(torch.autograd.Function):
         B, T = mixture.shape
         S, n_fft, hop = eng.cfg["n_src"], eng.cfg["n_fft"], eng.cfg["hop"]
         dev = mixture.device
-        ws = torch.empty(max(256, lib.tfl_mss_train_workspace_bytes(eng.plan, B, T)), dtype=torch.uint8, device=dev)
+        det = torch.are_deterministic_algorithms_enabled()
         shape = (S, B, T) if want_audio else (B, S, 1 + T // hop, n_fft // 2 + 1, 2)
         out = torch.empty(shape, dtype=torch.float32, device=dev)
         packed = eng.packed
-        with torch.cuda.device(dev):
+        with deterministic_option(det), torch.cuda.device(dev):
+            ws = torch.empty(max(256, lib.tfl_mss_train_workspace_bytes(eng.plan, B, T)), dtype=torch.uint8, device=dev)
             check(lib.tfl_mss_train_forward(eng.plan, packed.data_ptr(), mixture.data_ptr(), B, T,
                                             out.data_ptr() if want_audio else None,
                                             None if want_audio else out.data_ptr(), ws.data_ptr(), ws.numel(),
                                             _stream()))
-        ctx.eng, ctx.want_audio, ctx.shape = eng, want_audio, (B, T)
+        ctx.eng, ctx.want_audio, ctx.shape, ctx.deterministic = eng, want_audio, (B, T), det
         ctx.save_for_backward(packed, ws, *params)
         return out
 
@@ -102,7 +107,7 @@ class MSSFunction(torch.autograd.Function):
         grads = torch.empty(_grad_layout(eng)[2], dtype=torch.float32, device=dev)
         d_out = d_out.to(torch.float32).contiguous()
         d_mix = torch.empty((B, T), dtype=torch.float32, device=dev) if ctx.needs_input_grad[1] else None
-        with torch.cuda.device(dev):
+        with deterministic_option(ctx.deterministic), torch.cuda.device(dev):
             check(eng.lib.tfl_mss_train_backward(eng.plan, packed.data_ptr(), _weights_array(raw), len(raw),
                                                  d_out.data_ptr() if ctx.want_audio else None,
                                                  None if ctx.want_audio else d_out.data_ptr(), B, T, grads.data_ptr(),
@@ -120,13 +125,14 @@ class SeparatorFunction(torch.autograd.Function):
         lib = eng.lib
         B, Tf, F, _ = spec_ri.shape
         dev = spec_ri.device
-        ws = torch.empty(max(256, lib.tfl_sep_train_workspace_bytes(eng.plan, B, Tf, F)), dtype=torch.uint8, device=dev)
+        det = torch.are_deterministic_algorithms_enabled()
         est = torch.empty((B, eng.cfg["n_src"], Tf, F, 2), dtype=torch.float32, device=dev)
         packed = eng.packed
-        with torch.cuda.device(dev):
+        with deterministic_option(det), torch.cuda.device(dev):
+            ws = torch.empty(max(256, lib.tfl_sep_train_workspace_bytes(eng.plan, B, Tf, F)), dtype=torch.uint8, device=dev)
             check(lib.tfl_sep_train_forward(eng.plan, packed.data_ptr(), spec_ri.data_ptr(), B, Tf, F, est.data_ptr(),
                                             ws.data_ptr(), ws.numel(), _stream()))
-        ctx.eng = eng
+        ctx.eng, ctx.deterministic = eng, det
         ctx.save_for_backward(spec_ri, packed, ws, *params)
         return est
 
@@ -142,7 +148,7 @@ class SeparatorFunction(torch.autograd.Function):
         args = (eng.plan, packed.data_ptr(), _weights_array(raw), len(raw), d_est.data_ptr(), spec_ri.data_ptr(), B, Tf, F,
                 grads.data_ptr(), ws.data_ptr(), ws.numel(), _stream())
         d_spec = torch.empty_like(spec_ri) if ctx.needs_input_grad[1] else None
-        with torch.cuda.device(spec_ri.device):
+        with deterministic_option(ctx.deterministic), torch.cuda.device(spec_ri.device):
             if d_spec is None:
                 check(eng.lib.tfl_sep_train_backward(*args))
             else:
@@ -169,11 +175,12 @@ class BSFunction(torch.autograd.Function):
         dev = ri.device
         wbuf, tab = model._bs_packed(dev)
         packed = eng.packed
-        ws = torch.empty(max(256, lib.tfl_sep_train_workspace_bytes(eng.plan, B, T, nb)), dtype=torch.uint8, device=dev)
+        det = torch.are_deterministic_algorithms_enabled()
         x0 = torch.empty((B, T, nb, Cd), dtype=torch.float32, device=dev)
         x1 = torch.empty_like(x0)
         est = torch.empty((B, S, M, T, F, 2), dtype=torch.float32, device=dev)
-        with torch.cuda.device(dev):
+        with deterministic_option(det), torch.cuda.device(dev):
+            ws = torch.empty(max(256, lib.tfl_sep_train_workspace_bytes(eng.plan, B, T, nb)), dtype=torch.uint8, device=dev)
             check(lib.tfl_bs_band_split(ri.data_ptr(), B, M, T, F, Cd, nb, wmax, tab.data_ptr(), wbuf.data_ptr(),
                                         x0.data_ptr(), _stream()))
             check(lib.tfl_blocks_train_forward(eng.plan, packed.data_ptr(), x0.data_ptr(), B, T, nb, x1.data_ptr(),
@@ -181,7 +188,7 @@ class BSFunction(torch.autograd.Function):
             check(lib.tfl_bs_band_decode(x1.data_ptr(), ri.data_ptr(), B, M, T, F, Cd, nb, S, tab.data_ptr(),
                                          wbuf.data_ptr(), est.data_ptr(), 1 if model.masking else 0, _stream()))
         del x0
-        ctx.eng, ctx.model_cfg = eng, (nb, Cd, S, wmax, bool(model.masking), len(eng.keys))
+        ctx.eng, ctx.model_cfg, ctx.deterministic = eng, (nb, Cd, S, wmax, bool(model.masking), len(eng.keys)), det
         ctx.band_map = model._bs_pack[3]
         ctx.save_for_backward(ri, packed, wbuf, tab, ws, x1, *params)
         return est
@@ -204,7 +211,7 @@ class BSFunction(torch.autograd.Function):
         raw = _raw(blk_params)
         n_bws = lib.tfl_bs_band_bwd_workspace_bytes(B, M, T, F, Cd, nb, S, wmax)
         bws = torch.empty(max(256, n_bws), dtype=torch.uint8, device=dev)
-        with torch.cuda.device(dev):
+        with deterministic_option(ctx.deterministic), torch.cuda.device(dev):
             check(lib.tfl_bs_band_decode_bwd(x1.data_ptr(), ri.data_ptr(), d_est.data_ptr(), B, M, T, F, Cd, nb, S, wmax,
                                              tab.data_ptr(), wbuf.data_ptr(), 1 if masking else 0, dx1.data_ptr(),
                                              gw.data_ptr(), bws.data_ptr(), bws.numel(), _stream()))

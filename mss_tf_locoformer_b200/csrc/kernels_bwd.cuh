@@ -12,7 +12,11 @@
 //   istft_bwd_kernel          adjoint of iSTFT + overlap-add + envelope normalisation
 //   loss kernels              SI-SDR + L1 + log-magnitude STFT loss and its gradient w.r.t. the separated audio
 //   sqnorm / adamw            gradient clipping (torch.nn.utils.clip_grad_norm_) and torch.optim.AdamW
-// All fp32 on CUDA cores, accumulations over rows through fp32 atomics (order-dependent in the last bits).
+//   ordered_sum_kernel        second stage of every reduction of the deterministic mode
+// All fp32 on CUDA cores.  By default the reductions over rows end in fp32 / double atomics, so their result depends on
+// the order the blocks finish in (the last bits).  The kernels with a `DET` template switch (TFL_OPT_DETERMINISTIC)
+// instead reduce inside a block in a fixed order and store one partial per block or row split; ordered_sum_kernel adds the
+// partials in index order.  Every other reduction here is atomic-free and already fixed-order.
 #pragma once
 #include "kernels_f32.cuh"
 
@@ -76,18 +80,52 @@ struct EpiSwiGLUBwd {
   }
 };
 
+// ---- deterministic mode: out[b][i] += sum over r = 0 .. n_rows - 1 of part[b][r][i], r ascending ----------------------
+// One kernel serves every reduction of the mode: the per-split slabs of the weight-gradient GEMMs, the per-block partials
+// of the bias, gamma, decoder and encoder gradients (float) and of the encoder statistics and loss rows (double).
+template <class T>
+__global__ void __launch_bounds__(256) ordered_sum_kernel(const T* __restrict__ part, int n_rows, long long row_stride,
+                                                          long long width, long long part_bstride, T* __restrict__ out,
+                                                          long long out_bstride) {
+  const T* pb = part + (size_t)blockIdx.y * part_bstride;
+  T* ob = out + (size_t)blockIdx.y * out_bstride;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < width; i += (long long)gridDim.x * blockDim.x) {
+    T acc = 0;
+    for (int r = 0; r < n_rows; ++r) acc += pb[(size_t)r * row_stride + i];
+    ob[i] += acc;
+  }
+}
+
 // ---- weight gradients ---------------------------------------------------------------------------------------------
 // out[tap][i][n] += sum over rows r = (s, j), j in [0, Sout): A[s, j + tap - padL, i] * B[s, j, n]
 // (A rows outside [0, Sin) are the zero padding).  Grid: x = tap * tiles_i * tiles_n, y = row splits; every block
-// reduces its slice of the rows into a 128 x 128 register-tiled accumulator and adds it to `out` with fp32 atomics.
+// reduces its slice of the rows into a 128 x 128 register-tiled accumulator and adds it to `out` with fp32 atomics, or
+// (DET) stores it into the slab of its split, out[split][tap][i][n], for ordered_sum_kernel.  Every split owns at least
+// one row, so the splits of a tile together write every slab entry.
 struct TapWgrad {
   const float* A; SeqMap amap; int Sin, padL, taps, Kc;
   const float* B; SeqMap bmap; int Sout, N;
   long long R;            // rows = nseq * Sout
-  float* out;             // [taps][Kc][N]
+  float* out;             // [taps][Kc][N]  (DET: [splits][taps][Kc][N])
   long long rows_per_split;
 };
 
+// the epilogue store of the three weight-gradient kernels: slab base of (split, tap), then add or store
+template <bool DET>
+__device__ __forceinline__ float* wgrad_out(const TapWgrad& p, int tap) {
+  return p.out + ((size_t)(DET ? blockIdx.y * p.taps : 0) + tap) * p.Kc * p.N;
+}
+template <bool DET>
+__device__ __forceinline__ void wgrad_put(float* o, float v) {
+  if (DET) *o = v; else atomicAdd(o, v);
+}
+template <bool DET>
+__device__ __forceinline__ void wgrad_put2(float* o, float v0, float v1) {   // o 8-byte aligned (n even, N % 4 == 0)
+  if (DET) *reinterpret_cast<float2*>(o) = make_float2(v0, v1);
+  else { atomicAdd(o, v0); atomicAdd(o + 1, v1); }
+}
+
+template <bool DET>
 __global__ void __launch_bounds__(256) tap_wgrad_kernel(TapWgrad p) {
   __shared__ float As[2][GBK][GBM];
   __shared__ float Bs[2][GBK][GBN];
@@ -148,7 +186,7 @@ __global__ void __launch_bounds__(256) tap_wgrad_kernel(TapWgrad p) {
     __syncthreads();
     cur ^= 1;
   }
-  float* o = p.out + (size_t)tap * p.Kc * p.N;
+  float* o = wgrad_out<DET>(p, tap);
 #pragma unroll
   for (int i = 0; i < 8; ++i) {
     const int ii = i0 + ty * 8 + i;
@@ -156,20 +194,23 @@ __global__ void __launch_bounds__(256) tap_wgrad_kernel(TapWgrad p) {
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
       const int nn = n0 + tx * 8 + j;
-      if (nn < p.N) atomicAdd(&o[(size_t)ii * p.N + nn], acc[i][j]);
+      if (nn < p.N) wgrad_put<DET>(&o[(size_t)ii * p.N + nn], acc[i][j]);
     }
   }
 }
 
 // out[n] += sum over rows (s, j) of B[s, j, n]   (bias gradients).  One thread per column group of 4, blocks over rows.
+// DET: the rows_par row lanes of a block keep their sums apart in shared memory ([rows_par][N]), are added in lane order,
+// and the block stores its column sums into out[block][n] for ordered_sum_kernel.
+template <bool DET>
 __global__ void __launch_bounds__(256) colsum_kernel(const float* __restrict__ B, SeqMap bmap, int Sout, int N, long long R,
                                                      float* __restrict__ out) {
-  extern __shared__ float cs_sm[];   // [N]
-  for (int i = threadIdx.x; i < N; i += blockDim.x) cs_sm[i] = 0.f;
-  __syncthreads();
+  extern __shared__ float cs_sm[];   // [N]  (DET: [rows_par][N])
   const int n4 = N >> 2;
   const int lanes = n4 < 256 ? n4 : 256;             // threads along the columns
   const int rows_par = 256 / lanes;                  // rows handled in parallel by one block
+  for (int i = threadIdx.x; i < (DET ? rows_par : 1) * N; i += blockDim.x) cs_sm[i] = 0.f;
+  __syncthreads();
   const int col = (threadIdx.x % lanes), rsub = threadIdx.x / lanes;
   // every block owns a contiguous run of rows; (sequence, position) is carried along it instead of divided out per row
   const long long chunk = (R + gridDim.x - 1) / gridDim.x;
@@ -189,19 +230,34 @@ __global__ void __launch_bounds__(256) colsum_kernel(const float* __restrict__ B
           base = bmap.base(s);
         }
       }
-      atomicAdd(&cs_sm[4 * c4], acc.x); atomicAdd(&cs_sm[4 * c4 + 1], acc.y);
-      atomicAdd(&cs_sm[4 * c4 + 2], acc.z); atomicAdd(&cs_sm[4 * c4 + 3], acc.w);
+      if (DET) {
+        *reinterpret_cast<float4*>(&cs_sm[(size_t)rsub * N + 4 * c4]) = acc;
+      } else {
+        atomicAdd(&cs_sm[4 * c4], acc.x); atomicAdd(&cs_sm[4 * c4 + 1], acc.y);
+        atomicAdd(&cs_sm[4 * c4 + 2], acc.z); atomicAdd(&cs_sm[4 * c4 + 3], acc.w);
+      }
     }
   }
   __syncthreads();
-  for (int i = threadIdx.x; i < N; i += blockDim.x) atomicAdd(&out[i], cs_sm[i]);
+  if (DET) {
+    for (int i = threadIdx.x; i < N; i += blockDim.x) {
+      float s = 0.f;
+      for (int q = 0; q < rows_par; ++q) s += cs_sm[(size_t)q * N + i];
+      out[(size_t)blockIdx.x * N + i] = s;
+    }
+  } else {
+    for (int i = threadIdx.x; i < N; i += blockDim.x) atomicAdd(&out[i], cs_sm[i]);
+  }
 }
 
 // ---- RMSGroupNorm backward (models/mss_tflocoformer.py:682-706) ----------------------------------------------------
 // y_c = x_c / r * gamma_c,  r = ||x_g|| / sqrt(D) + eps.  With dot = sum_c gamma_c dy_c x_c over the group:
 //   dx_c = gamma_c dy_c / r - x_c * dot / (r^2 * ||x_g|| * sqrt(D)),   dgamma_c += dy_c x_c / r.
 // dx_total (in place) += dx: the incoming gradient of the residual stream passes through unchanged.
-template <int W>
+// DET: the launcher makes the pair stride a multiple of G, so every slot of W threads keeps one group's channels in
+// registers; the slots' sums meet in shared memory ([slots][D]) and are added in slot order into dgamma[block][C], the
+// block's partial for ordered_sum_kernel.
+template <int W, bool DET>
 __global__ void __launch_bounds__(256) rms_group_norm_bwd_kernel(const float* __restrict__ x, const float* __restrict__ dy,
                                                                  float* __restrict__ dx_total, long long rows, int C, int G,
                                                                  const float* __restrict__ gamma, float eps,
@@ -257,6 +313,20 @@ __global__ void __launch_bounds__(256) rms_group_norm_bwd_kernel(const float* __
         atomicAdd(&gsm[c + 2], d.z * v.z * inv_r); atomicAdd(&gsm[c + 3], d.w * v.w * inv_r);
       }
     }
+  }
+  if (DET) {
+    const int slots = blockDim.x / W, slot = threadIdx.x / W;
+    __syncthreads();
+    if (sub < lanes) *reinterpret_cast<float4*>(&gsm[slot * D + (sub << 2)]) = ga;   // zero for a slot without rows
+    __syncthreads();
+    for (int i = threadIdx.x; i < C; i += blockDim.x) {
+      const int grp = i / D;
+      float s = 0.f;
+      for (int q = 0; q < slots; ++q)
+        if ((int)(((long long)blockIdx.x * slots + q) % G) == grp) s += gsm[q * D + i - grp * D];
+      dgamma[(size_t)blockIdx.x * C + i] = s;
+    }
+    return;
   }
   if (c_fixed >= 0) {
     atomicAdd(&gsm[c_fixed], ga.x); atomicAdd(&gsm[c_fixed + 1], ga.y);
@@ -445,6 +515,8 @@ __global__ void __launch_bounds__(256) dec_dgrad_kernel(const float* __restrict_
 
 // wgrad: gw[dt*3+df][o][c] += sum_{b, tt, ff} x[tt, ff][c] * dEst[o][tt-1+dt, ff-1+df]
 // Thread = channel (blockDim.x == C rounded up to a warp multiple), blocks over positions; 72 accumulators per thread.
+// DET: gw is [blocks][9][8][C]; each block stores its sums there for ordered_sum_kernel.
+template <bool DET>
 __global__ void __launch_bounds__(256) dec_wgrad_kernel(const float* __restrict__ x, const float* __restrict__ dest, int n_frames,
                                                         int n_freq, int C, int n_out, long long n_pos,
                                                         float* __restrict__ gw /*[9][8][C]*/) {
@@ -477,8 +549,12 @@ __global__ void __launch_bounds__(256) dec_wgrad_kernel(const float* __restrict_
     }
   }
   if (c < C) {
+    float* g = gw + (DET ? (size_t)blockIdx.x * 72 * C : 0);
 #pragma unroll
-    for (int i = 0; i < 72; ++i) atomicAdd(&gw[(size_t)i * C + c], acc[i]);
+    for (int i = 0; i < 72; ++i) {
+      if (DET) g[(size_t)i * C + c] = acc[i];
+      else atomicAdd(&g[(size_t)i * C + c], acc[i]);
+    }
   }
 }
 
@@ -502,6 +578,9 @@ __global__ void __launch_bounds__(256) dec_bias_grad_kernel(const float* __restr
 // ---- encoder backward: y = gLN(conv(spec)) = (v - mean) * rstd * gw_c + gb_c, statistics over (C, Tf, F) per sample ------
 // pass 1: dgw_c += sum dy * vhat, dgb_c += sum dy, per-sample S1 = sum dy * gw_c, S2 = sum dy * gw_c * vhat (double).
 // v is the conv output (pre-norm), recomputed by enc_conv_kernel.  Thread = channel, blocks over positions.
+// DET: per (sample, block) partials -- dgw [B][blocks][2C] = (dgw, dgb), sums [B][blocks][2] -- for ordered_sum_kernel
+// (dgb unused).
+template <bool DET>
 __global__ void __launch_bounds__(256) enc_gln_bwd_stats_kernel(const float* __restrict__ v, const float* __restrict__ dy,
                                                                 long long per_sample_pos, int C, const float* __restrict__ stats,
                                                                 const float* __restrict__ gw, float* __restrict__ dgw,
@@ -519,7 +598,11 @@ __global__ void __launch_bounds__(256) enc_gln_bwd_stats_kernel(const float* __r
       s1 += (double)(d * w); s2 += (double)(d * w * vh);
     }
   }
-  if (c < C) { atomicAdd(&dgw[c], a_w); atomicAdd(&dgb[c], a_b); }
+  const size_t part = (size_t)b * gridDim.x + blockIdx.x;
+  if (c < C) {
+    if (DET) { dgw[part * 2 * C + c] = a_w; dgw[part * 2 * C + C + c] = a_b; }
+    else { atomicAdd(&dgw[c], a_w); atomicAdd(&dgb[c], a_b); }
+  }
   __shared__ double r1[256], r2[256];
   r1[threadIdx.x] = s1; r2[threadIdx.x] = s2;
   __syncthreads();
@@ -527,12 +610,16 @@ __global__ void __launch_bounds__(256) enc_gln_bwd_stats_kernel(const float* __r
     if (threadIdx.x < o && threadIdx.x + o < blockDim.x) { r1[threadIdx.x] += r1[threadIdx.x + o]; r2[threadIdx.x] += r2[threadIdx.x + o]; }
     __syncthreads();
   }
-  if (threadIdx.x == 0) { atomicAdd(&sums[b * 2], r1[0]); atomicAdd(&sums[b * 2 + 1], r2[0]); }
+  if (threadIdx.x == 0) {
+    if (DET) { sums[part * 2] = r1[0]; sums[part * 2 + 1] = r2[0]; }
+    else { atomicAdd(&sums[b * 2], r1[0]); atomicAdd(&sums[b * 2 + 1], r2[0]); }
+  }
 }
 
 // pass 2: dv = rstd * (dy * gw_c - S1 / n - vhat * S2 / n);  conv weight gradient
 //   gwc[(dt*3+df)][ci][c] += sum_pos dv[pos][c] * spec[t+dt-1, f+df-1][ci],  gbc[c] += sum dv.
-template <int CIN>
+// DET: gwc is [B][blocks][9 CIN + 1][C] (the bias row last; gbc unused), stored per (sample, block) for ordered_sum_kernel.
+template <int CIN, bool DET>
 __global__ void __launch_bounds__(256) enc_wgrad_kernel(const float* __restrict__ v, const float* __restrict__ dy,
                                                         const float* __restrict__ spec, int n_frames, int n_freq, int C,
                                                         const float* __restrict__ stats, const double* __restrict__ sums,
@@ -572,7 +659,12 @@ __global__ void __launch_bounds__(256) enc_wgrad_kernel(const float* __restrict_
       }
     }
   }
-  if (c < C) {
+  if (c < C && DET) {
+    float* g = gwc + ((size_t)b * gridDim.x + blockIdx.x) * (9 * CIN + 1) * C;
+#pragma unroll
+    for (int i = 0; i < 9 * CIN; ++i) g[(size_t)i * C + c] = acc[i];
+    g[(size_t)9 * CIN * C + c] = bacc;
+  } else if (c < C) {
 #pragma unroll
     for (int i = 0; i < 9 * CIN; ++i) atomicAdd(&gwc[(size_t)i * C + c], acc[i]);
     atomicAdd(&gbc[c], bacc);
@@ -743,6 +835,8 @@ __global__ void sisdr_coef_kernel(const double* __restrict__ s5, LossCfg cfg, fl
 
 // log-magnitude L1 between the loss spectrograms: partial sums per row, and dE written over E:
 //   dE = w_spec / count * sign(log1p|E| - log1p|T|) / (1 + |E|) * E / |E|     (count = batch * bins * frames, per source)
+// DET: sum_rows is [rows][blocks], one partial per block for ordered_sum_kernel.
+template <bool DET>
 __global__ void __launch_bounds__(256) spec_loss_kernel(float2* __restrict__ E, const float2* __restrict__ T, long long per_row,
                                                         float coef, double* __restrict__ sum_rows /*[rows]*/) {
   const int row = blockIdx.y;
@@ -762,7 +856,10 @@ __global__ void __launch_bounds__(256) spec_loss_kernel(float2* __restrict__ E, 
   red[threadIdx.x] = acc;
   __syncthreads();
   for (int o = 128; o > 0; o >>= 1) { if (threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o]; __syncthreads(); }
-  if (threadIdx.x == 0) atomicAdd(&sum_rows[row], red[0]);
+  if (threadIdx.x == 0) {
+    if (DET) sum_rows[(size_t)row * gridDim.x + blockIdx.x] = red[0];
+    else atomicAdd(&sum_rows[row], red[0]);
+  }
 }
 
 // adjoint of the rfft of one windowed frame: frames[row][t][m] = w[m] * sum_k (dRe_k cos(2 pi k m / N) - dIm_k sin(...))
@@ -789,7 +886,8 @@ __global__ void __launch_bounds__(256) stft_adj_frames_kernel(const float2* __re
 }
 
 // d loss / d est[row][n] = SI-SDR (affine) + L1 sign + the adjoint of (reflect pad -> frame) applied to `frames`;
-// also accumulates sum |est - tgt| per row for the reported L1 loss.
+// also accumulates sum |est - tgt| per row for the reported L1 loss (DET: l1_rows is [rows][blocks] of block partials).
+template <bool DET>
 __global__ void __launch_bounds__(256) loss_grad_kernel(const float* __restrict__ est, const float* __restrict__ tgt,
                                                         const float* __restrict__ coef, const float* __restrict__ frames,
                                                         LossCfg cfg, float* __restrict__ dest, double* __restrict__ l1_rows) {
@@ -830,7 +928,10 @@ __global__ void __launch_bounds__(256) loss_grad_kernel(const float* __restrict_
   red[threadIdx.x] = l1;
   __syncthreads();
   for (int o = 128; o > 0; o >>= 1) { if (threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o]; __syncthreads(); }
-  if (threadIdx.x == 0) atomicAdd(&l1_rows[row], red[0]);
+  if (threadIdx.x == 0) {
+    if (DET) l1_rows[(size_t)row * gridDim.x + blockIdx.x] = red[0];
+    else atomicAdd(&l1_rows[row], red[0]);
+  }
 }
 
 // loss_out[0] = total, then per source {si_sdr, l1, spectral} (means as the reference reports them)

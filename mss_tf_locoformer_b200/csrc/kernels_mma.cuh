@@ -133,6 +133,7 @@ __global__ void __launch_bounds__(256, 2) tap_gemm_mma_kernel(TapGemm p, Epi epi
   }
 }
 
+template <bool DET>
 __global__ void __launch_bounds__(256, 2) tap_wgrad_mma_kernel(TapWgrad p) {
   __shared__ __align__(16) uint32_t As[2][MMA_BK][MMA_PITCH];
   __shared__ __align__(16) uint32_t Bs[2][MMA_BK][MMA_PITCH];
@@ -207,7 +208,7 @@ __global__ void __launch_bounds__(256, 2) tap_wgrad_mma_kernel(TapWgrad p) {
     __syncthreads();
     cur ^= 1;
   }
-  float* o = p.out + (size_t)tap * p.Kc * p.N;
+  float* o = wgrad_out<DET>(p, tap);
 #pragma unroll
   for (int i = 0; i < 4; ++i)
 #pragma unroll
@@ -217,10 +218,7 @@ __global__ void __launch_bounds__(256, 2) tap_wgrad_mma_kernel(TapWgrad p) {
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
         const int nn = n0 + wn * 32 + j * 8 + 2 * t;
-        if (nn < p.N) {
-          atomicAdd(&o[(size_t)ii * p.N + nn], acc[i][j][2 * h]);
-          atomicAdd(&o[(size_t)ii * p.N + nn + 1], acc[i][j][2 * h + 1]);
-        }
+        if (nn < p.N) wgrad_put2<DET>(&o[(size_t)ii * p.N + nn], acc[i][j][2 * h], acc[i][j][2 * h + 1]);
       }
     }
 }
@@ -358,6 +356,7 @@ __global__ void __launch_bounds__(256, 2) tap_gemm_bf16_kernel(TapGemm p, Epi ep
   }
 }
 
+template <bool DET>
 __global__ void __launch_bounds__(256, 2) tap_wgrad_bf16_kernel(TapWgrad p) {
   __shared__ __align__(16) __nv_bfloat16 As[2][32][BF_BP];   // [k = row][m = i]
   __shared__ __align__(16) __nv_bfloat16 Bs[2][32][BF_BP];   // [k = row][n]
@@ -440,7 +439,7 @@ __global__ void __launch_bounds__(256, 2) tap_wgrad_bf16_kernel(TapWgrad p) {
     __syncthreads();
     cur ^= 1;
   }
-  float* o = p.out + (size_t)tap * p.Kc * p.N;
+  float* o = wgrad_out<DET>(p, tap);
 #pragma unroll
   for (int i = 0; i < 4; ++i)
 #pragma unroll
@@ -450,10 +449,7 @@ __global__ void __launch_bounds__(256, 2) tap_wgrad_bf16_kernel(TapWgrad p) {
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
         const int nn = n0 + wn * 32 + j * 8 + 2 * t;
-        if (nn < p.N) {
-          atomicAdd(&o[(size_t)ii * p.N + nn], acc[i][j][2 * h]);
-          atomicAdd(&o[(size_t)ii * p.N + nn + 1], acc[i][j][2 * h + 1]);
-        }
+        if (nn < p.N) wgrad_put2<DET>(&o[(size_t)ii * p.N + nn], acc[i][j][2 * h], acc[i][j][2 * h + 1]);
       }
     }
 }

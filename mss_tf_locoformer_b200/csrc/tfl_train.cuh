@@ -57,12 +57,99 @@ struct TrainWs {
   size_t ckpt, dx, dxn, scratch, lse, dbuf, nat, wt, dest, audio, daudio;
   size_t s5, stats_scratch, coef, loss_rows, l1_rows, spec_rows, ltab_tw, ltab_win, lspec_e, lspec_t, lframes, enc_sums;
   size_t dspec, adj_frames;  // saved mode with T > 0 (the MSS autograd pair): d spec [B][Tf][F][2], frame adjoints [B][Tf][n_fft]
+  size_t det;                // TFL_OPT_DETERMINISTIC: partials of the reductions, sized for the largest one (0 = option off)
   size_t total;
   // inside `scratch` (FFN and attention backward never overlap in time)
   size_t dg, hid2, dh;       // FFN: dG, recomputed hidden, dH
   size_t dO, dqkv_h, dqkv;   // attention
   int n_sub, l_frames, l_freq;
 };
+
+// ---- deterministic mode (TFL_OPT_DETERMINISTIC) ----------------------------------------------------------------------
+// Every reduction over rows of the backward pass stores one partial per block or row split and ordered_sum_kernel adds
+// them in index order.  Its grids are sized for a 148-SM B200 whatever the device, so the order of each of these sums is a
+// function of the shapes alone (DESIGN.md section 8b names the one forward reduction that still follows the SM count).
+constexpr int DET_SMS = 148;
+
+static float* det_ptr(const TrainWs& tw, char* wsp) { return tw.det != 0 ? (float*)(wsp + tw.det) : nullptr; }
+
+template <class T>
+static int ordered_sum(const T* part, int n_rows, long long row_stride, long long width, T* out, cudaStream_t st,
+                       int batch = 1, long long part_bstride = 0, long long out_bstride = 0) {
+  long long blocks = (width + 255) / 256;
+  if (blocks > DET_SMS * 8) blocks = DET_SMS * 8;
+  ordered_sum_kernel<T><<<dim3((unsigned)blocks, batch), 256, 0, st>>>(part, n_rows, row_stride, width, part_bstride, out,
+                                                                       out_bstride);
+  TFL_LAUNCH_CHECK();
+  return 0;
+}
+
+// Row splits of a weight-gradient GEMM (sets rows_per_split): about four CTAs per SM, at least 256 rows per split.
+static long long wgrad_splits(TapWgrad& g, int sm_count) {
+  const int tiles = g.taps * ((g.Kc + GBM - 1) / GBM) * ((g.N + GBN - 1) / GBN);
+  long long splits = ((long long)sm_count * 4 + tiles - 1) / tiles;
+  const long long max_splits = (g.R + 255) / 256;
+  if (splits > max_splits) splits = max_splits;
+  if (splits < 1) splits = 1;
+  if (splits > 65535) splits = 65535;
+  g.rows_per_split = ((g.R + splits - 1) / splits + 31) / 32 * 32;
+  return (g.R + g.rows_per_split - 1) / g.rows_per_split;
+}
+static long long wgrad_slab_bytes(int taps, int Kc, int N, long long R) {
+  TapWgrad g{};
+  g.taps = taps; g.Kc = Kc; g.N = N; g.R = R;
+  return wgrad_splits(g, DET_SMS) * taps * Kc * N * (long long)sizeof(float);
+}
+static long long colsum_blocks(long long R, int sm_count) {
+  const long long blocks = (R + 63) / 64;
+  return blocks > (long long)sm_count * 4 ? (long long)sm_count * 4 : blocks;
+}
+// RMSGroupNorm backward: threads per (row, group) pair W and the block count; `det` rounds the blocks up to a multiple of
+// G, which makes every slot of W threads keep one group for all of its rows
+static long long norm_bwd_blocks(long long rows, int C, int G, int sm_count, bool det, int* W_out) {
+  const int lanes = (C / G) / 4;
+  int W = 1;
+  while (W < lanes) W <<= 1;
+  *W_out = W;
+  const long long per_block = 256 / W;
+  long long blocks = (rows * G + per_block - 1) / per_block;
+  if (blocks > (long long)sm_count * 8) blocks = (long long)sm_count * 8;
+  if (blocks < 1) blocks = 1;
+  return det ? (blocks + G - 1) / G * G : blocks;
+}
+constexpr int DET_DEC_BLOCKS = DET_SMS * 4, DET_ENC_BLOCKS = DET_SMS * 2, DET_LOSS_BLOCKS = DET_SMS;
+
+// The partials of the largest reduction of a step of this shape: every weight-gradient slab, bias, gamma, decoder and
+// encoder partial, and (loss_rows > 0) the loss row sums.  One buffer serves them all: they are consumed in stream order.
+static size_t det_scratch_bytes(const tfl_plan* pl, int B, int Tf, int F, int loss_rows) {
+  const tfl_config& c = pl->cfg;
+  const int C = c.emb_dim, A = c.attention_dim, K = c.conv_kernel;
+  const long long rows = (long long)B * Tf * F;
+  long long need = 0;
+  auto at_least = [&](long long bytes) { if (bytes > need) need = bytes; };
+  for (int axis = 0; axis < 2; ++axis) {
+    const long long S = axis == TFL_AXIS_FREQ ? F : Tf, nseq = rows / S, rows1 = nseq * (S + K - 1);
+    for (int j = 0; j < pl->n_ffn; ++j) {
+      const int H = j == 0 ? c.ffn_hidden0 : c.ffn_hidden1;
+      at_least(wgrad_slab_bytes(K, H, C, rows));
+      at_least(wgrad_slab_bytes(K, C, 2 * H, rows1));
+      at_least(colsum_blocks(rows, DET_SMS) * C * 4);
+      at_least(colsum_blocks(rows1, DET_SMS) * 2 * H * 4);
+    }
+    at_least(wgrad_slab_bytes(1, C, A, rows));
+    at_least(wgrad_slab_bytes(1, 3 * A, C, rows));
+  }
+  int W;
+  at_least(norm_bwd_blocks(rows, C, c.num_groups, DET_SMS, true, &W) * C * 4);
+  if (c.enc_in_ch > 0) {
+    at_least((long long)DET_DEC_BLOCKS * 72 * C * 4);
+    const long long enc_parts = (long long)B * DET_ENC_BLOCKS;
+    at_least(align_up(enc_parts * 2 * C * 4) + enc_parts * 2 * 8);          // enc_gln_bwd_stats_kernel
+    at_least(enc_parts * (9 * c.enc_in_ch + 1) * C * 4);                     // enc_wgrad_kernel
+  }
+  at_least((long long)loss_rows * DET_SMS * 2 * 8);                          // loss_grad_kernel (spec_loss_kernel: half)
+  return (size_t)need;
+}
 
 // (B, Tf, F) size the network buffers; T (audio samples, 0 = stage-level use) and the loss STFT size the rest.
 // `saved`: the checkpoint slots of one saved forward, without the loss buffers.  T = 0: the separators' frames-only
@@ -125,50 +212,66 @@ static TrainWs plan_train_ws(const tfl_plan* pl, int B, int Tf, int F, int T, in
     w.lspec_t = take(rows * w.l_frames * w.l_freq * sizeof(float2));
     w.lframes = take(rows * w.l_frames * (size_t)l_fft * sizeof(float));
   }
+  w.det = tfl_option(TFL_OPT_DETERMINISTIC) ? take(det_scratch_bytes(pl, B, Tf, F, saved ? 0 : (int)rows)) : 0;
   w.total = off;
   return w;
 }
 
-static int wgrad_launch(TapWgrad g, int sm_count, cudaStream_t st) {
+// The three launchers below add into `out` / `dgamma` with atomics, or -- with `det` (the partials buffer of the
+// deterministic mode) -- store per-split / per-block partials there and add them in index order.
+static int wgrad_launch(TapWgrad g, int sm_count, cudaStream_t st, float* det = nullptr) {
   TFL_CHECK(g.Kc % 4 == 0 && g.N % 4 == 0, "weight-gradient GEMM needs Kc %% 4 == 0 and N %% 4 == 0 (Kc %d N %d)", g.Kc, g.N);
   const int tiles = g.taps * ((g.Kc + GBM - 1) / GBM) * ((g.N + GBN - 1) / GBN);
-  long long splits = ((long long)sm_count * 4 + tiles - 1) / tiles;
-  const long long max_splits = (g.R + 255) / 256;
-  if (splits > max_splits) splits = max_splits;
-  if (splits < 1) splits = 1;
-  if (splits > 65535) splits = 65535;
-  g.rows_per_split = ((g.R + splits - 1) / splits + 31) / 32 * 32;
-  splits = (g.R + g.rows_per_split - 1) / g.rows_per_split;
-  if (g_gemm_mode == 2) tap_wgrad_bf16_kernel<<<dim3((unsigned)tiles, (unsigned)splits), 256, 0, st>>>(g);
-  else if (g_gemm_mode == 1) tap_wgrad_mma_kernel<<<dim3((unsigned)tiles, (unsigned)splits), 256, 0, st>>>(g);
-  else tap_wgrad_kernel<<<dim3((unsigned)tiles, (unsigned)splits), 256, 0, st>>>(g);
+  const long long splits = wgrad_splits(g, det != nullptr ? DET_SMS : sm_count);
+  const dim3 grid((unsigned)tiles, (unsigned)splits);
+  if (det != nullptr) {
+    float* out = g.out;
+    g.out = det;
+    if (g_gemm_mode == 2) tap_wgrad_bf16_kernel<true><<<grid, 256, 0, st>>>(g);
+    else if (g_gemm_mode == 1) tap_wgrad_mma_kernel<true><<<grid, 256, 0, st>>>(g);
+    else tap_wgrad_kernel<true><<<grid, 256, 0, st>>>(g);
+    TFL_LAUNCH_CHECK();
+    const long long slab = (long long)g.taps * g.Kc * g.N;
+    return ordered_sum(det, (int)splits, slab, slab, out, st);
+  }
+  if (g_gemm_mode == 2) tap_wgrad_bf16_kernel<false><<<grid, 256, 0, st>>>(g);
+  else if (g_gemm_mode == 1) tap_wgrad_mma_kernel<false><<<grid, 256, 0, st>>>(g);
+  else tap_wgrad_kernel<false><<<grid, 256, 0, st>>>(g);
   TFL_LAUNCH_CHECK();
   return 0;
 }
 
-static int colsum_launch(const float* Bm, SeqMap bmap, int Sout, int N, long long R, float* out, int sm_count, cudaStream_t st) {
+static int colsum_launch(const float* Bm, SeqMap bmap, int Sout, int N, long long R, float* out, int sm_count, cudaStream_t st,
+                         float* det = nullptr) {
   TFL_CHECK(N % 4 == 0, "column sum needs N %% 4 == 0");
-  long long blocks = (R + 63) / 64;
-  if (blocks > (long long)sm_count * 4) blocks = (long long)sm_count * 4;
-  colsum_kernel<<<(unsigned)blocks, 256, (size_t)N * sizeof(float), st>>>(Bm, bmap, Sout, N, R, out);
+  const long long blocks = colsum_blocks(R, det != nullptr ? DET_SMS : sm_count);
+  if (det != nullptr) {
+    const int lanes = N / 4 < 256 ? N / 4 : 256;
+    colsum_kernel<true><<<(unsigned)blocks, 256, (size_t)(256 / lanes) * N * sizeof(float), st>>>(Bm, bmap, Sout, N, R, det);
+    TFL_LAUNCH_CHECK();
+    return ordered_sum(det, (int)blocks, N, N, out, st);
+  }
+  colsum_kernel<false><<<(unsigned)blocks, 256, (size_t)N * sizeof(float), st>>>(Bm, bmap, Sout, N, R, out);
   TFL_LAUNCH_CHECK();
   return 0;
 }
 
 static int norm_bwd_launch(const float* x, const float* dy, float* dx_total, long long rows, int C, int G, const float* gamma,
-                           float eps, float* dgamma, int sm_count, cudaStream_t st) {
-  const int lanes = (C / G) / 4;
-  int W = 1;
-  while (W < lanes) W <<= 1;
+                           float eps, float* dgamma, int sm_count, cudaStream_t st, float* det = nullptr) {
+  int W;
+  const long long blocks = norm_bwd_blocks(rows, C, G, det != nullptr ? DET_SMS : sm_count, det != nullptr, &W);
   TFL_CHECK(W <= 32, "emb_dim/num_groups > 128 is not supported");
-  const long long pairs = rows * G;
-  const long long per_block = 256 / W;
-  long long blocks = (pairs + per_block - 1) / per_block;
-  long long cap = (long long)sm_count * 8;
-  if (blocks > cap) blocks = cap;
-  if (blocks < 1) blocks = 1;
+  if (det != nullptr) {
+    const size_t slots_d = (size_t)(256 / W) * (C / G);
+    const size_t sm = (slots_d > (size_t)C ? slots_d : (size_t)C) * sizeof(float);
+#define NB_CASE(w) case w: rms_group_norm_bwd_kernel<w, true><<<(int)blocks, 256, sm, st>>>(x, dy, dx_total, rows, C, G, gamma, eps, det); break;
+    switch (W) { NB_CASE(1) NB_CASE(2) NB_CASE(4) NB_CASE(8) NB_CASE(16) NB_CASE(32) }
+#undef NB_CASE
+    TFL_LAUNCH_CHECK();
+    return ordered_sum(det, (int)blocks, C, C, dgamma, st);
+  }
   const size_t sm = (size_t)C * sizeof(float);
-#define NB_CASE(w) case w: rms_group_norm_bwd_kernel<w><<<(int)blocks, 256, sm, st>>>(x, dy, dx_total, rows, C, G, gamma, eps, dgamma); break;
+#define NB_CASE(w) case w: rms_group_norm_bwd_kernel<w, false><<<(int)blocks, 256, sm, st>>>(x, dy, dx_total, rows, C, G, gamma, eps, dgamma); break;
   switch (W) { NB_CASE(1) NB_CASE(2) NB_CASE(4) NB_CASE(8) NB_CASE(16) NB_CASE(32) }
 #undef NB_CASE
   TFL_LAUNCH_CHECK();
@@ -216,6 +319,7 @@ static int ffn_backward(const tfl_plan* pl, const char* packed, int layer, int a
   float* hid = (float*)(wsp + tw.hid2);
   float* dh = (float*)(wsp + tw.dh);
   float* nat = (float*)(wsp + tw.nat);
+  float* det = det_ptr(tw, wsp);
   float* nat_w1 = nat, *nat_b1 = nat_w1 + (size_t)K * C * 2 * H, *nat_w2 = nat_b1 + 2 * H;
   float* w2t = (float*)(wsp + tw.wt);                 // [K][C][H]:   w2t[t][c][h]  = deconv1d.weight[h][c][t]
   float* w1t = w2t + (size_t)K * C * H;               // [K][2H][C]:  w1t[t][2h+q][c] = conv1d.weight[q*H+h][c][K-1-t]
@@ -235,18 +339,18 @@ static int ffn_backward(const tfl_plan* pl, const char* packed, int layer, int a
   if (gemm_launch(g1, EpiSwiGLUBwd{dg, hid, dh, H}, st)) return -1;
   // transposed-conv weights: nat_w2[k'][h][c] = sum hid[s, i + k'][h] * dY[s, i][c];  bias: sum dY
   TapWgrad gw2{hid, hmap, S + K - 1, 0, K, H, dx, xmap, S, C, (long long)nseq * S, nat_w2, 0};
-  if (wgrad_launch(gw2, pl->sm_count, st)) return -1;
-  if (colsum_launch(dx, xmap, S, C, (long long)nseq * S, gp.b2[j], pl->sm_count, st)) return -1;
+  if (wgrad_launch(gw2, pl->sm_count, st, det)) return -1;
+  if (colsum_launch(dx, xmap, S, C, (long long)nseq * S, gp.b2[j], pl->sm_count, st, det)) return -1;
   // conv1d weights: nat_w1[k][c][n] = sum xn[s, j' + k - (K-1)][c] * dH[s, j'][n];  bias: sum dH
   TapWgrad gw1{xn, xmap, S, K - 1, K, C, dh, h2map, S + K - 1, 2 * H, rows1, nat_w1, 0};
-  if (wgrad_launch(gw1, pl->sm_count, st)) return -1;
-  if (colsum_launch(dh, h2map, S + K - 1, 2 * H, rows1, nat_b1, pl->sm_count, st)) return -1;
+  if (wgrad_launch(gw1, pl->sm_count, st, det)) return -1;
+  if (colsum_launch(dh, h2map, S + K - 1, 2 * H, rows1, nat_b1, pl->sm_count, st, det)) return -1;
   // dxn[s, i] = sum_t dH[s, i + t] . w1t[t]
   TapGemm gx{dh, h2map, S + K - 1, S, 0, K, 2 * H, w1t, nullptr, C, (long long)nseq * S};
   if (gemm_launch(gx, EpiStoreMap{dxn, xmap}, st)) return -1;
   // through the norm, into the residual gradient
   if (norm_bwd_launch(x_in, dxn, dx, rows, C, c.num_groups, (const float*)(packed + f.gamma), c.eps, gp.ffn_gamma[j],
-                      pl->sm_count, st)) return -1;
+                      pl->sm_count, st, det)) return -1;
   // natural -> reference layouts
   permute(nat_w1, gp.w1[j], 2, H, C, K, 1, 2, 2 * H, (long long)C * 2 * H, 0, -1, st);       // conv1d.weight [2H, C, K]
   permute(nat_b1, gp.b1[j], 1, 1, 2, H, 0, 0, 1, 2, 0, -1, st);                              // conv1d.bias [2H]
@@ -275,6 +379,7 @@ static int attn_backward(const tfl_plan* pl, const char* packed, int layer, int 
   float* dqkv_h = (float*)(wsp + tw.dqkv_h);
   float* dqkv = (float*)(wsp + tw.dqkv);
   float* dxn = (float*)(wsp + tw.dxn);
+  float* det = det_ptr(tw, wsp);
   const SeqMap xmap = make_seq_map(axis, d.Tf, d.F, C);
   const SeqMap omap = make_dense_map((long long)L * A, A);
   const SeqMap qmap = make_dense_map((long long)L * 3 * A, 3 * A);
@@ -285,7 +390,7 @@ static int attn_backward(const tfl_plan* pl, const char* packed, int layer, int 
   if (gemm_launch(g_do, EpiStoreDense{dO}, st)) return -1;
   // dWo[c][a] = sum_r dY[r][c] * o[r][a]
   TapWgrad gwo{dx, xmap, L, 0, 1, C, o, omap, L, A, (long long)nseq * L, gp.wo, 0};
-  if (wgrad_launch(gwo, pl->sm_count, st)) return -1;
+  if (wgrad_launch(gwo, pl->sm_count, st, det)) return -1;
   const size_t per = (size_t)nseq * heads * L * hd;
   const float scale = 1.0f / sqrtf((float)hd);
   if (g_gemm_tf32 && hd % 2 == 0 && hd > 8 && hd <= 32) {   // tensor-core form (tf32 mma.sync), 64 rows per block
@@ -328,12 +433,12 @@ static int attn_backward(const tfl_plan* pl, const char* packed, int layer, int 
   }
   // dWqkv[n][c] = sum_r dQKV[r][n] * xn[r][c]   (qkv.weight is [3A, C])
   TapWgrad gwq{dqkv, qmap, L, 0, 1, 3 * A, xn, xmap, L, C, (long long)nseq * L, gp.wqkv, 0};
-  if (wgrad_launch(gwq, pl->sm_count, st)) return -1;
+  if (wgrad_launch(gwq, pl->sm_count, st, det)) return -1;
   // dxn = dQKV . Wqkv   (qkv.weight [3A, C] is exactly [Kc = 3A][N = C])
   TapGemm g_dx{dqkv, qmap, L, L, 0, 1, 3 * A, rp.wqkv, nullptr, C, (long long)nseq * L};
   if (gemm_launch(g_dx, EpiStoreMap{dxn, xmap}, st)) return -1;
   return norm_bwd_launch(x_in, dxn, dx, rows, C, c.num_groups, (const float*)(packed + p.attn_gamma), c.eps, gp.attn_gamma,
-                         pl->sm_count, st);
+                         pl->sm_count, st, det);
 }
 
 // sub-blocks of the network in forward order: (layer, axis, kind) with kind 0 / 1 = ffn index, 2 = attention
@@ -431,8 +536,14 @@ static int dec_backward(const tfl_plan* pl, const char* pk, const GradLayout& gl
   float* dx = (float*)(wsp + tw.dx);
   // weights: natural layout [9][8][C] -> deconv.weight [C, 2S, 3, 3]
   TFL_CUDA(cudaMemsetAsync(nat, 0, ((size_t)9 * 8 * C + 8) * sizeof(float), st));
-  dec_wgrad_kernel<<<pl->sm_count * 4, cthreads, 0, st>>>(x, dest, d.Tf, d.F, C, 2 * S, (long long)N, nat);
-  TFL_LAUNCH_CHECK();
+  if (float* det = det_ptr(tw, wsp)) {
+    dec_wgrad_kernel<true><<<DET_DEC_BLOCKS, cthreads, 0, st>>>(x, dest, d.Tf, d.F, C, 2 * S, (long long)N, det);
+    TFL_LAUNCH_CHECK();
+    if (ordered_sum(det, DET_DEC_BLOCKS, (long long)72 * C, (long long)72 * C, nat, st)) return -1;
+  } else {
+    dec_wgrad_kernel<false><<<pl->sm_count * 4, cthreads, 0, st>>>(x, dest, d.Tf, d.F, C, 2 * S, (long long)N, nat);
+    TFL_LAUNCH_CHECK();
+  }
   permute(nat, grads + gl.off[n_w - 2], C, 2 * S, 3, 3, 1, C, (long long)3 * 8 * C, (long long)8 * C, 0, -1, st);
   dec_bias_grad_kernel<<<2 * S, 256, 0, st>>>(dest, d.B, S, (long long)d.Tf * d.F, grads + gl.off[n_w - 1]);
   TFL_LAUNCH_CHECK();
@@ -465,12 +576,29 @@ static int enc_backward(const tfl_plan* pl, const char* pk, const GradLayout& gl
   TFL_LAUNCH_CHECK();
   TFL_CUDA(cudaMemsetAsync(sums, 0, (size_t)B * 2 * sizeof(double), st));
   TFL_CUDA(cudaMemsetAsync(nat, 0, ((size_t)18 * C + C) * sizeof(float), st));
-  enc_gln_bwd_stats_kernel<<<dim3(pl->sm_count * 2, B), cthreads, 0, st>>>(v, dx, (long long)Tf * F, C, stats, (const float*)(pk + pl->lay.gln_w),
-                                                                         grads + gl.off[2], grads + gl.off[3], sums);
-  TFL_LAUNCH_CHECK();
-  enc_wgrad_kernel<2><<<dim3(pl->sm_count * 2, B), cthreads, 0, st>>>(v, dx, spec, Tf, F, C, stats, sums, (const float*)(pk + pl->lay.gln_w),
-                                                                    nat, nat + (size_t)18 * C);
-  TFL_LAUNCH_CHECK();
+  if (float* det = det_ptr(tw, wsp)) {
+    // (dgw, dgb) partials [B][blocks][2C], then the statistics partials [B][blocks][2] in double
+    const long long parts = (long long)B * DET_ENC_BLOCKS;
+    double* sums_part = (double*)((char*)det + align_up((size_t)parts * 2 * C * sizeof(float)));
+    const dim3 grid(DET_ENC_BLOCKS, B);
+    enc_gln_bwd_stats_kernel<true><<<grid, cthreads, 0, st>>>(v, dx, (long long)Tf * F, C, stats, (const float*)(pk + pl->lay.gln_w),
+                                                              det, nullptr, sums_part);
+    TFL_LAUNCH_CHECK();
+    if (ordered_sum(det, (int)parts, 2LL * C, (long long)C, grads + gl.off[2], st)) return -1;
+    if (ordered_sum(det + C, (int)parts, 2LL * C, (long long)C, grads + gl.off[3], st)) return -1;
+    if (ordered_sum(sums_part, DET_ENC_BLOCKS, 2LL, 2LL, sums, st, B, 2LL * DET_ENC_BLOCKS, 2LL)) return -1;
+    enc_wgrad_kernel<2, true><<<grid, cthreads, 0, st>>>(v, dx, spec, Tf, F, C, stats, sums, (const float*)(pk + pl->lay.gln_w),
+                                                         det, nullptr);
+    TFL_LAUNCH_CHECK();
+    if (ordered_sum(det, (int)parts, 19LL * C, 19LL * C, nat, st)) return -1;   // [18 C] weights, then [C] bias, as in nat
+  } else {
+    enc_gln_bwd_stats_kernel<false><<<dim3(pl->sm_count * 2, B), cthreads, 0, st>>>(v, dx, (long long)Tf * F, C, stats, (const float*)(pk + pl->lay.gln_w),
+                                                                                    grads + gl.off[2], grads + gl.off[3], sums);
+    TFL_LAUNCH_CHECK();
+    enc_wgrad_kernel<2, false><<<dim3(pl->sm_count * 2, B), cthreads, 0, st>>>(v, dx, spec, Tf, F, C, stats, sums, (const float*)(pk + pl->lay.gln_w),
+                                                                               nat, nat + (size_t)18 * C);
+    TFL_LAUNCH_CHECK();
+  }
   // natural [9][ci][C] -> conv.0.weight [C, ci, 3, 3]
   permute(nat, grads + gl.off[0], 1, C, 2, 9, 0, 1, C, (long long)2 * C, 0, -1, st);
   permute(nat + (size_t)18 * C, grads + gl.off[1], 1, 1, 1, C, 0, 0, 0, 1, 0, -1, st);
@@ -630,6 +758,7 @@ int tfl_train_forward_backward(const tfl_plan* pl, const void* packed, const flo
   float* audio = (float*)(wsp + tw.audio);
   float* daudio = (float*)(wsp + tw.daudio);
   float* dest = (float*)(wsp + tw.dest);
+  float* det = det_ptr(tw, wsp);
   TFL_CUDA(cudaMemsetAsync(grads, 0, (size_t)gl.total * sizeof(float), st));
 
   // ---------------- forward ----------------
@@ -678,15 +807,29 @@ int tfl_train_forward_backward(const tfl_plan* pl, const void* packed, const flo
     TFL_LAUNCH_CHECK();
     const long long per_row = (long long)tw.l_frames * tw.l_freq;
     spec_count = (long long)B * per_row;
-    spec_loss_kernel<<<dim3(pl->sm_count, rows), 256, 0, st>>>(se, stt, per_row, loss->spectral_weight / (float)spec_count, spec_rows);
-    TFL_LAUNCH_CHECK();
+    if (det != nullptr) {
+      double* part = (double*)det;
+      spec_loss_kernel<true><<<dim3(DET_LOSS_BLOCKS, rows), 256, 0, st>>>(se, stt, per_row, loss->spectral_weight / (float)spec_count, part);
+      TFL_LAUNCH_CHECK();
+      if (ordered_sum(part, DET_LOSS_BLOCKS, 1LL, 1LL, spec_rows, st, rows, (long long)DET_LOSS_BLOCKS, 1LL)) return -1;
+    } else {
+      spec_loss_kernel<false><<<dim3(pl->sm_count, rows), 256, 0, st>>>(se, stt, per_row, loss->spectral_weight / (float)spec_count, spec_rows);
+      TFL_LAUNCH_CHECK();
+    }
     TFL_CUDA(opt_in_smem(stft_adj_frames_kernel, fsm));
     stft_adj_frames_kernel<<<dim3(tw.l_frames, rows), 256, fsm, st>>>(se, l_fft, lc.l_log, tw.l_frames, ltw, lwin, (float*)(wsp + tw.lframes));
     TFL_LAUNCH_CHECK();
     frames = (const float*)(wsp + tw.lframes);
   }
-  loss_grad_kernel<<<dim3(pl->sm_count * 2, rows), 256, 0, st>>>(audio, targets, coef, frames, lc, daudio, l1_rows);
-  TFL_LAUNCH_CHECK();
+  if (det != nullptr) {
+    double* part = (double*)det;
+    loss_grad_kernel<true><<<dim3(DET_LOSS_BLOCKS * 2, rows), 256, 0, st>>>(audio, targets, coef, frames, lc, daudio, part);
+    TFL_LAUNCH_CHECK();
+    if (ordered_sum(part, DET_LOSS_BLOCKS * 2, 1LL, 1LL, l1_rows, st, rows, (long long)DET_LOSS_BLOCKS * 2, 1LL)) return -1;
+  } else {
+    loss_grad_kernel<false><<<dim3(pl->sm_count * 2, rows), 256, 0, st>>>(audio, targets, coef, frames, lc, daudio, l1_rows);
+    TFL_LAUNCH_CHECK();
+  }
   loss_finish_kernel<<<1, 32, 0, st>>>(loss_rows, l1_rows, spec_on ? spec_rows : nullptr, lc, spec_count, loss_out);
   TFL_LAUNCH_CHECK();
 

@@ -10,6 +10,10 @@ Arithmetic (``tfl_debug_set_option(TFL_OPT_TRAIN_MODE, m)``): 0 = exact fp32 on 
 1 = tf32 ``mma.sync`` GEMMs, 2 (default) = forward of the sub-blocks on the bf16 tcgen05 inference kernels and bf16 / tf32
 ``mma.sync`` backward (DESIGN.md section 8b).  Dropout is not applied (parity is defined for p = 0): a model built with
 ``dropout > 0`` is refused.
+
+Under ``torch.use_deterministic_algorithms(True)`` (read at every ``forward_backward`` / ``step``) the backward pass
+reduces in a fixed order (``TFL_OPT_DETERMINISTIC``), so the same step from the same state gives bitwise-identical
+gradients, and clipping and AdamW, which are fixed-order already, keep them so.  The all-reduce across ranks is NCCL's.
 """
 import ctypes as C
 from typing import Dict, Optional, Union
@@ -17,7 +21,7 @@ from typing import Dict, Optional, Union
 import torch
 
 from . import _lib
-from ._lib import TflLossConfig, check
+from ._lib import TflLossConfig, check, deterministic_option
 from .engine import _require_cuda, _stream
 from .modules import SOURCE_NAMES
 
@@ -105,15 +109,16 @@ class Trainer:
         if tuple(targets.shape) != (S, B, T):
             raise ValueError(f"targets must be [{S}, {B}, {T}] (sources, batch, samples), got {tuple(targets.shape)}")
         eng = self.model._ready()
-        key = (B, T)
-        if self._ws_key != key:
-            n = self.lib.tfl_train_workspace_bytes(eng.plan, B, T, self.loss_cfg.spec_n_fft, self.loss_cfg.spec_hop)
-            self._ws = None
-            self._ws = torch.empty(n, dtype=torch.uint8, device=mixture.device)
-            self._ws_key = key
+        det = torch.are_deterministic_algorithms_enabled()
         loss = torch.empty(1 + 3 * S, dtype=torch.float32, device=mixture.device)
         audio = torch.empty((S, B, T), dtype=torch.float32, device=mixture.device) if want_audio else None
-        with torch.cuda.device(mixture.device):
+        with deterministic_option(det), torch.cuda.device(mixture.device):
+            key = (B, T, det)
+            if self._ws_key != key:
+                n = self.lib.tfl_train_workspace_bytes(eng.plan, B, T, self.loss_cfg.spec_n_fft, self.loss_cfg.spec_hop)
+                self._ws = None
+                self._ws = torch.empty(n, dtype=torch.uint8, device=mixture.device)
+                self._ws_key = key
             check(self.lib.tfl_train_forward_backward(
                 eng.plan, eng.packed.data_ptr(), self._weights_array(), len(self.tensors), mixture.data_ptr(),
                 targets.data_ptr(), B, T, C.byref(self.loss_cfg), self.grads.data_ptr(), loss.data_ptr(),
@@ -208,11 +213,11 @@ def _stage_setup(model, x_in: torch.Tensor):
 def ffn_backward(model, layer: int, axis: int, index: int, x_in: torch.Tensor, dy: torch.Tensor):
     """x_out = x_in + FFN(norm(x_in)) along ``axis`` on channels-last [B, Tf, F, C]: returns (dL/dx_in, grad_of(key))."""
     _require_cuda(x_in, "x_in")
-    lib, eng, arr, n, ws, grads, grad_of, staged = _stage_setup(model, x_in)
     B, Tf, F, _ = x_in.shape
     dx = dy.detach().to(torch.float32).contiguous().clone()
     xc = x_in.detach().to(torch.float32).contiguous()
-    with torch.cuda.device(x_in.device):
+    with deterministic_option(torch.are_deterministic_algorithms_enabled()), torch.cuda.device(x_in.device):
+        lib, eng, arr, n, ws, grads, grad_of, staged = _stage_setup(model, x_in)
         check(lib.tfl_conv_swiglu_ffn_bwd(eng.plan, eng.packed.data_ptr(), arr, n, layer, axis, index, xc.data_ptr(),
                                           dx.data_ptr(), B, Tf, F, grads.data_ptr(), ws.data_ptr(), ws.numel(), _stream()))
         torch.cuda.synchronize()
@@ -222,11 +227,11 @@ def ffn_backward(model, layer: int, axis: int, index: int, x_in: torch.Tensor, d
 def attn_backward(model, layer: int, axis: int, x_in: torch.Tensor, dy: torch.Tensor):
     """x_out = x_in + MHSA(norm(x_in)) along ``axis``: returns (dL/dx_in, grad_of(key))."""
     _require_cuda(x_in, "x_in")
-    lib, eng, arr, n, ws, grads, grad_of, staged = _stage_setup(model, x_in)
     B, Tf, F, _ = x_in.shape
     dx = dy.detach().to(torch.float32).contiguous().clone()
     xc = x_in.detach().to(torch.float32).contiguous()
-    with torch.cuda.device(x_in.device):
+    with deterministic_option(torch.are_deterministic_algorithms_enabled()), torch.cuda.device(x_in.device):
+        lib, eng, arr, n, ws, grads, grad_of, staged = _stage_setup(model, x_in)
         check(lib.tfl_rope_attn_bwd(eng.plan, eng.packed.data_ptr(), arr, n, layer, axis, xc.data_ptr(), dx.data_ptr(),
                                     B, Tf, F, grads.data_ptr(), ws.data_ptr(), ws.numel(), _stream()))
         torch.cuda.synchronize()
