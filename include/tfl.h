@@ -24,6 +24,15 @@ typedef struct CUstream_st* tfl_stream_t; /* == cudaStream_t */
 
 #define TFL_PRECISION_FP32 0 /* CUDA-core fp32 everywhere: the <=1e-4 / >=70 dB parity mode            */
 #define TFL_PRECISION_BF16 1 /* tcgen05 bf16 MMAs with fp32 TMEM accumulation, fp32 residual stream      */
+/* TFL_PRECISION_TF32: what the reference computes on a GPU without autocast (cuDNN convolutions in TF32 by default,
+ * matmuls and SDPA in fp32):
+ *   STFT, iSTFT, RMSGroupNorm, gLN statistics, RoPE, residual stream   exact fp32, as in TFL_PRECISION_FP32
+ *   encoder conv + gLN, decoder                                        the tf32 mma.sync kernels of TFL_PRECISION_BF16
+ *   ConvSwiGLU FFN (conv1d + SwiGLU, transposed conv + bias + residual) tcgen05 kind::tf32: operands rounded to tf32
+ *                                                                      (cvt.rna), fp32 accumulation in TMEM
+ *   q|k|v projection + RoPE, attention, head merge + residual          exact fp32, as in TFL_PRECISION_FP32
+ * Workspace layout and size are those of TFL_PRECISION_FP32. */
+#define TFL_PRECISION_TF32 2
 #define TFL_AXIS_FREQ 0      /* sequences run along F, one per (b, t)  -- freq_path                      */
 #define TFL_AXIS_TIME 1      /* sequences run along Tf, one per (b, f) -- frame_path                     */
 
@@ -81,7 +90,7 @@ int tfl_enc_conv_gln(const tfl_plan* plan, const void* packed, const float* spec
                      int n_freq, float* x, void* workspace, size_t ws_bytes, tfl_stream_t stream);
 /* The same stage in the arithmetic of `precision`: TFL_PRECISION_FP32 = tfl_enc_conv_gln; TFL_PRECISION_BF16 = the tf32
  * mma.sync encoder that tfl_forward / tfl_separator_forward run in bf16 mode (spectrogram and weights rounded to tf32,
- * fp32 sums, gLN statistics in double). */
+ * fp32 sums, gLN statistics in double); TFL_PRECISION_TF32 runs the same kernels as TFL_PRECISION_BF16. */
 int tfl_enc_conv_gln_mode(const tfl_plan* plan, const void* packed, const float* spec, int batch, int n_frames,
                           int n_freq, float* x, void* workspace, size_t ws_bytes, int precision, tfl_stream_t stream);
 /* :682-706.  x [rows, C] -> y [rows, C] with the gamma of (layer, axis, which) where
@@ -105,7 +114,8 @@ int tfl_rope_attn(const tfl_plan* plan, const void* packed, int layer, int axis,
 int tfl_dec_conv(const tfl_plan* plan, const void* packed, const float* x, int batch, int n_frames,
                  int n_freq, float* est, tfl_stream_t stream);
 /* The same stage in the arithmetic of `precision`: TFL_PRECISION_FP32 = tfl_dec_conv; TFL_PRECISION_BF16 = the tf32
- * mma.sync decoder that tfl_forward / tfl_separator_forward run in bf16 mode (operands rounded to tf32, fp32 sums). */
+ * mma.sync decoder that tfl_forward / tfl_separator_forward run in bf16 mode (operands rounded to tf32, fp32 sums);
+ * TFL_PRECISION_TF32 runs the same kernels as TFL_PRECISION_BF16. */
 int tfl_dec_conv_mode(const tfl_plan* plan, const void* packed, const float* x, int batch, int n_frames,
                       int n_freq, float* est, int precision, tfl_stream_t stream);
 /* :56-75, :239-250.  est [B, S, Tf, F, 2] -> audio [S, B, n_samples] (all sources, one launch). */
@@ -282,7 +292,9 @@ int tfl_debug_set_trace(void* device_buffer);
  * mode 0: D[128, N] = sum_{tap < taps} A[m + tap, :] . B[tap][n, :]   A [128 + taps - 1, Kd], B [taps, N, Kd]
  * mode 1: D[128, N] = A[m, :] . B[:, n]                               A [128, Kd], B [Kd, N] (N-contiguous)
  * mode 2: as mode 1 with A staged in TMEM (tcgen05.st) instead of shared memory; N <= 128, Kd <= 256
- * Operands are rounded to bf16, accumulation is fp32.  scratch: >= taps * N * Kd * 2 bytes. */
+ * Operands are rounded to bf16, accumulation is fp32.  scratch: >= taps * N * Kd * 2 bytes.
+ * mode 3: mode 0's row-shifted tap product in tcgen05 kind::tf32 through the tap-GEMM kernel of TFL_PRECISION_TF32's FFN
+ *         (operands rounded to tf32 with cvt.rna, fp32 accumulation; Kd % 8 == 0).  scratch: >= taps * N * Kd * 4 bytes. */
 int tfl_tc_selftest(const float* A, const float* B, float* D, void* scratch, int N, int Kd, int taps, int mode,
                     tfl_stream_t stream);
 

@@ -17,6 +17,7 @@
 #include "kernels_bs.cuh"
 #include "kernels_bwd.cuh"
 #include "kernels_mma.cuh"
+#include "kernels_tf32.cuh"
 
 namespace tfl {
 
@@ -286,7 +287,7 @@ static Workspace plan_workspace(const tfl_plan* pl, int B, int Tf, int F, int pr
   w.gln_part = take((size_t)B * w.gln_blocks * 2 * sizeof(double));
   w.gln_stats = take((size_t)B * 2 * sizeof(float));
   w.prefix = off;   // everything above is precision-independent (tfl_enc_conv_gln uses only this part)
-  if (precision == TFL_PRECISION_FP32) {   // CUDA-core path: normalised copy, hidden activation, q|k|v, attention output
+  if (precision == TFL_PRECISION_FP32 || precision == TFL_PRECISION_TF32) {   // normalised copy, hidden, q|k|v, attention output
     const size_t hid_rows_f = (size_t)B * Tf * (F + K - 1), hid_rows_t = (size_t)B * F * (Tf + K - 1);
     const size_t hid_rows = hid_rows_f > hid_rows_t ? hid_rows_f : hid_rows_t;
     w.xn = take(N * C * sizeof(float));
@@ -344,9 +345,10 @@ static int gemm_launch(const TapGemm& g, const Epi& epi, cudaStream_t st) {
 
 struct Dims { int B, Tf, F; };
 
+// tf32 = the same dataflow with both GEMMs on the tcgen05 kind::tf32 tap-GEMM (kernels_tf32.cuh)
 static int ffn_f32(const tfl_plan* pl, const char* packed, int layer, int axis, int j, float* x, Dims d,
-                   const Workspace& ws, char* wsp, cudaStream_t st) {
-  NvtxRange nvtx_range("tfl::conv_swiglu_ffn[fp32]");
+                   const Workspace& ws, char* wsp, cudaStream_t st, bool tf32 = false) {
+  NvtxRange nvtx_range(tf32 ? "tfl::conv_swiglu_ffn[tf32]" : "tfl::conv_swiglu_ffn[fp32]");
   const tfl_config& c = pl->cfg;
   const FfnPack& f = pl->lay.paths[(size_t)layer * 2 + axis].ffn[j];
   const int C = c.emb_dim, K = c.conv_kernel, H = f.hidden;
@@ -359,9 +361,13 @@ static int ffn_f32(const tfl_plan* pl, const char* packed, int layer, int axis, 
   const SeqMap xmap = make_seq_map(axis, d.Tf, d.F, C);
   TapGemm g1{xn, xmap, S, S + K - 1, K - 1, K, C, (const float*)(packed + f.w1), (const float*)(packed + f.b1),
              2 * H, (long long)nseq * (S + K - 1)};
-  if (gemm_launch(g1, EpiSwiGLU{hid, H}, st)) return -1;
   TapGemm g2{hid, make_dense_map((long long)(S + K - 1) * H, H), S + K - 1, S, 0, K, H,
              (const float*)(packed + f.w2), (const float*)(packed + f.b2), C, (long long)nseq * S};
+  if (tf32) {
+    if (tap_gemm_tf32_launch(g1, EpiSwiGLU{hid, H}, st)) return -1;
+    return tap_gemm_tf32_launch(g2, EpiResidual{x, xmap}, st);
+  }
+  if (gemm_launch(g1, EpiSwiGLU{hid, H}, st)) return -1;
   return gemm_launch(g2, EpiResidual{x, xmap}, st);
 }
 
@@ -519,7 +525,7 @@ static int path_forward(const tfl_plan* pl, const char* packed, int layer, int a
       float* t = *cur; *cur = *alt; *alt = t;
       return 0;
     }
-    return ffn_f32(pl, packed, layer, axis, j, *cur, d, ws, wsp, st);
+    return ffn_f32(pl, packed, layer, axis, j, *cur, d, ws, wsp, st, precision == TFL_PRECISION_TF32);
   };
   if (pl->cfg.macaron && ffn(1)) return -1;
   if (precision == TFL_PRECISION_BF16) {
@@ -545,7 +551,8 @@ static int blocks_forward(const tfl_plan* pl, const char* packed, float* x, Dims
 static int check_common(const tfl_plan* pl, const void* packed, int B, int Tf, int F, int precision) {
   TFL_CHECK(pl != nullptr && packed != nullptr, "null plan / packed weights");
   TFL_CHECK(B >= 1 && Tf >= 1 && F >= 1, "empty input (batch %d, frames %d, bins %d)", B, Tf, F);
-  TFL_CHECK(precision == TFL_PRECISION_FP32 || precision == TFL_PRECISION_BF16, "unknown precision %d", precision);
+  TFL_CHECK(precision == TFL_PRECISION_FP32 || precision == TFL_PRECISION_BF16 || precision == TFL_PRECISION_TF32,
+            "unknown precision %d", precision);
   if (ensure_device_ready()) return -1;
   return timeout_pending();
 }
@@ -586,7 +593,8 @@ int tfl_enc_conv_gln(const tfl_plan* pl, const void* packed, const float* spec, 
 }
 int tfl_enc_conv_gln_mode(const tfl_plan* pl, const void* packed, const float* spec, int B, int Tf, int F, float* x,
                           void* workspace, size_t ws_bytes, int precision, tfl_stream_t stream) {
-  TFL_CHECK(precision == TFL_PRECISION_FP32 || precision == TFL_PRECISION_BF16, "unknown precision %d", precision);
+  TFL_CHECK(precision == TFL_PRECISION_FP32 || precision == TFL_PRECISION_BF16 || precision == TFL_PRECISION_TF32,
+            "unknown precision %d", precision);
   return enc_conv_gln_any(pl, packed, spec, B, Tf, F, x, workspace, ws_bytes, precision, stream);
 }
 }  // extern "C"
@@ -606,7 +614,7 @@ static int enc_conv_gln_any(const tfl_plan* pl, const void* packed, const float*
   double* part = (double*)(wsp + ws.gln_part);
   float* stats = (float*)(wsp + ws.gln_stats);
   const size_t smem = ((size_t)9 * 2 * C + C) * sizeof(float);
-  if (precision == TFL_PRECISION_BF16 && C % 8 == 0) {   // tf32 mma.sync path, two passes (see enc_conv_mma_kernel)
+  if (precision != TFL_PRECISION_FP32 && C % 8 == 0) {   // bf16 and tf32 modes: tf32 mma.sync, two passes (enc_conv_mma_kernel)
     const size_t msm = ((size_t)24 * (C + 8) + 3 * C) * sizeof(float);
     TFL_CUDA(opt_in_smem(enc_conv_mma_kernel<2, 0>, msm));
     TFL_CUDA(opt_in_smem(enc_conv_mma_kernel<2, 1>, msm));
@@ -664,7 +672,7 @@ int tfl_conv_swiglu_ffn(const tfl_plan* pl, const void* packed, int layer, int a
     return 0;
   }
   return ffn_f32(pl, (const char*)packed, layer, axis, ffn_index, x, Dims{B, Tf, F}, ws, (char*)workspace,
-                 (cudaStream_t)stream);
+                 (cudaStream_t)stream, precision == TFL_PRECISION_TF32);
 }
 
 int tfl_conv_swiglu_ffn_out(const tfl_plan* pl, const void* packed, int layer, int axis, int ffn_index, const float* x,
@@ -681,7 +689,7 @@ int tfl_conv_swiglu_ffn_out(const tfl_plan* pl, const void* packed, int layer, i
   TFL_CUDA(cudaMemcpyAsync(y, x, (size_t)B * Tf * F * pl->cfg.emb_dim * sizeof(float), cudaMemcpyDeviceToDevice,
                            (cudaStream_t)stream));
   return ffn_f32(pl, (const char*)packed, layer, axis, ffn_index, y, Dims{B, Tf, F}, ws, (char*)workspace,
-                 (cudaStream_t)stream);
+                 (cudaStream_t)stream, precision == TFL_PRECISION_TF32);
 }
 
 int tfl_rope_attn(const tfl_plan* pl, const void* packed, int layer, int axis, float* x, int B, int Tf, int F,
@@ -697,11 +705,11 @@ int tfl_rope_attn(const tfl_plan* pl, const void* packed, int layer, int axis, f
 
 }  // extern "C"
 namespace tfl {
-// bf16 mode: tf32 mma.sync decoder (C % 16 == 0); fp32 mode and odd widths: the CUDA-core kernel (tfl_dec_conv)
+// bf16 and tf32 modes: tf32 mma.sync decoder (C % 16 == 0); fp32 mode and odd widths: the CUDA-core kernel (tfl_dec_conv)
 static int dec_conv_any(const tfl_plan* pl, const void* packed, const float* x, int B, int Tf, int F, float* est,
                         int precision, tfl_stream_t stream) {
   const int C = pl->cfg.emb_dim;
-  if (precision != TFL_PRECISION_BF16 || C % 16 != 0 || pl->cfg.n_src * 2 > 8) return tfl_dec_conv(pl, packed, x, B, Tf, F, est, stream);
+  if (precision == TFL_PRECISION_FP32 || C % 16 != 0 || pl->cfg.n_src * 2 > 8) return tfl_dec_conv(pl, packed, x, B, Tf, F, est, stream);
   NvtxRange nvtx_range("tfl::dec_conv[tf32]");
   if (check_common(pl, packed, B, Tf, F, precision)) return -1;
   if (C % 32 == 0 && C <= 128 && tfl_option(TFL_OPT_DEC_KERNEL) != 1) {
@@ -1049,6 +1057,10 @@ int tfl_debug_timeout(uint32_t* out5, int reset) {
 int tfl_tc_selftest(const float* A, const float* B, float* D, void* scratch, int N, int Kd, int taps, int mode,
                     tfl_stream_t stream) {
   TFL_CHECK(A && B && D && scratch, "null argument");
+  if (mode == 3) {
+    TFL_CHECK(N % 16 == 0 && N <= 256 && Kd % 8 == 0 && taps >= 1 && taps <= 8, "selftest shape");
+    return tf32_selftest(A, B, D, scratch, N, Kd, taps, (cudaStream_t)stream);
+  }
   return tc_selftest(A, B, D, scratch, N, Kd, taps, mode, (cudaStream_t)stream);
 }
 

@@ -11,7 +11,7 @@ import torch
 from . import _lib
 from ._lib import TflConfig, check
 
-PRECISIONS = {"fp32": 0, "bf16": 1}
+PRECISIONS = {"fp32": 0, "bf16": 1, "tf32": 2}
 AXIS = {"freq": 0, "time": 1}
 
 
@@ -268,13 +268,13 @@ def segment_ola(seg_audio: torch.Tensor, seg_index0: int, n_seg_total: int, trac
 
 def tc_selftest(A: torch.Tensor, B: torch.Tensor, taps: int, mode: int) -> torch.Tensor:
     """Diagnostic for the tcgen05 plumbing (tfl_tc_selftest).  mode 0: A [128+taps-1, Kd], B [taps, N, Kd];
-    mode 1: A [128, Kd], B [Kd, N].  Returns D [128, N] fp32."""
+    mode 1: A [128, Kd], B [Kd, N]; mode 3: as mode 0 in tcgen05 kind::tf32.  Returns D [128, N] fp32."""
     _require_cuda(A, "A")
     lib = _lib.load()
     Kd = A.shape[1]
     N = B.shape[1] if mode == 0 else B.shape[1]
     D = torch.empty((128, N), dtype=torch.float32, device=A.device)
-    scratch = torch.empty(max(256, taps * N * Kd * 2), dtype=torch.uint8, device=A.device)
+    scratch = torch.empty(max(256, taps * N * Kd * (4 if mode == 3 else 2)), dtype=torch.uint8, device=A.device)
     with torch.cuda.device(A.device):
         check(lib.tfl_tc_selftest(A.contiguous().data_ptr(), B.contiguous().data_ptr(), D.data_ptr(),
                                   scratch.data_ptr(), N, Kd, taps, mode, _stream()))

@@ -15,7 +15,7 @@ from .modules import (MSSTransform, RotaryEmbedding, TFLocoformerBlock, SOURCE_N
 class _SeparatorBase(nn.Module):
     """Shared plumbing: engine creation, lazy weight packing, sub-module call sites."""
 
-    precision: Optional[str] = None  # None = follow torch.autocast (bf16) else fp32; or "fp32" / "bf16"
+    precision: Optional[str] = None  # None = follow torch.autocast (bf16) else fp32; or "fp32" / "bf16" / "tf32"
     # True: in training mode with grad enabled, forward builds an autograd graph over the parameters and, for
     # TFLocoformerMSS and TFLocoformerSeparator, the input (autograd.py).  training.Trainer does not need it.
     differentiable: bool = False

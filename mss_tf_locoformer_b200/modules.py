@@ -19,8 +19,9 @@ SOURCE_NAMES = ["vocals", "drums", "bass", "other"]  # models/mss_tflocoformer.p
 
 
 def _resolve_precision(owner) -> int:
-    """'fp32' | 'bf16' | None (auto: bf16 iff the caller is inside torch.autocast(cuda, bfloat16),
-    which is how the reference enters its bf16 mode -- SURVEY.md F9)."""
+    """'fp32' | 'bf16' | 'tf32' | None (auto: bf16 iff the caller is inside torch.autocast(cuda, bfloat16),
+    which is how the reference enters its bf16 mode -- SURVEY.md F9; fp32 otherwise).  'tf32' is opt-in only: it is
+    never chosen from torch.backends.cudnn.allow_tf32, whose default is True."""
     p = getattr(owner, "precision", None)
     if p is None:
         auto = torch.is_autocast_enabled("cuda") and torch.get_autocast_dtype("cuda") == torch.bfloat16

@@ -3,7 +3,7 @@
 
     python -m mss_tf_locoformer_b200.separate --input song.wav --checkpoint model.pt [--config cfg.yaml]
         [--output_dir ./separated] [--device cuda] [--sample_rate 44100] [--seed 42]
-        [--segment 6.0] [--batch 8] [--precision bf16|fp32]
+        [--segment 6.0] [--batch 8] [--precision bf16|fp32|tf32]
 
 Same flags, same checkpoint / YAML handling, same mono down-mix, same stereo duplication and peak normalisation
 of the outputs as /root/reference/inference/separate.py:28-193 (`load_model` :79-116, `separate_audio` :119-169) and
@@ -40,7 +40,7 @@ def parse_args(argv=None):
     p.add_argument("--seed", type=int, default=42, help="Random seed")
     p.add_argument("--segment", type=float, default=6.0, help="Segment length in seconds (0 = whole track in one forward)")
     p.add_argument("--batch", type=int, default=8, help="Segments per forward")
-    p.add_argument("--precision", type=str, default="bf16", choices=["bf16", "fp32"])
+    p.add_argument("--precision", type=str, default="bf16", choices=["bf16", "fp32", "tf32"])
     return p.parse_args(argv)
 
 
