@@ -139,6 +139,14 @@ int tfl_separator_forward(const tfl_plan* plan, const void* packed, const float*
  * [track_origin, track_origin + n_track) of the full track (a rank's own range plus its halo; 0 = whole track). */
 int tfl_segment_ola(const float* seg_audio, int n_src, int batch, int seg_len, int seg_index0,
                     int n_seg_total, float* track, int64_t n_track, int64_t track_origin, tfl_stream_t stream);
+/* The same stitch at any hop (0 < hop < seg_len, segment i starts at i * hop) and over several channels:
+ * track[rows, channels, n_track] += sum_i w_i * seg_audio[rows, batch * channels, seg_len] / E, where row
+ * b * channels + c of seg_audio is channel c of segment seg_index0 + b, and E(t) = sum of the windows of all
+ * n_seg_total segments covering sample t (1 at hop = seg_len / 2).  One thread per output sample, no atomics:
+ * bitwise reproducible for a given batch.  `track` holds samples [track_origin, track_origin + n_track). */
+int tfl_segment_ola_hop(const float* seg_audio, int rows, int channels, int batch, int seg_len, int hop,
+                        int seg_index0, int n_seg_total, float* track, int64_t n_track, int64_t track_origin,
+                        tfl_stream_t stream);
 
 /* evaluation/metrics.py:14-168 on the device.  est, tgt [rows, n] fp32 -> out5 [rows][5] double =
  * {sum e, sum t, sum e^2, sum t^2, sum e*t}: SI-SDR, SDR and the file's "SAR" / "SIR" are closed forms of these sums

@@ -11,6 +11,7 @@ from .modules import (  # noqa: F401
     ConvDeconv1d, LocoformerBlock, MSSTransform, MultiHeadSelfAttention, RMSGroupNorm, RotaryEmbedding,
     SwiGLUConvDeconv1d, TFLocoformerBlock,
 )
-from .engine import Engine, segment_ola  # noqa: F401
+from .engine import Engine, segment_ola, segment_ola_hop  # noqa: F401
 
-__all__ = ["TFLocoformerMSS", "TFLocoformerSeparator", "BSLocoformerSeparator", "strip_prefix", "Engine", "segment_ola"]
+__all__ = ["TFLocoformerMSS", "TFLocoformerSeparator", "BSLocoformerSeparator", "strip_prefix", "Engine", "segment_ola",
+           "segment_ola_hop"]

@@ -49,6 +49,7 @@ SIGNATURES = {  # name -> (restype, argtypes); must list every symbol of include
     "tfl_forward": (_I, [_P, _P, _P, _I, _I, _P, _P, _P, _Z, _I, _P]),
     "tfl_separator_forward": (_I, [_P, _P, _P, _I, _I, _I, _P, _P, _Z, _I, _P]),
     "tfl_segment_ola": (_I, [_P, _I, _I, _I, _I, _I, _P, _L, _L, _P]),
+    "tfl_segment_ola_hop": (_I, [_P, _I, _I, _I, _I, _I, _I, _I, _P, _L, _L, _P]),
     "tfl_pair_stats": (_I, [_P, _P, _I, _L, _P, _P, _Z, _P]),
     "tfl_bs_band_split": (_I, [_P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P, _P]),
     "tfl_bs_band_decode": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P, _I, _P]),

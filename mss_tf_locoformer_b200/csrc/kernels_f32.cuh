@@ -992,6 +992,43 @@ __global__ void __launch_bounds__(256) segment_ola_kernel(const float* __restric
 }
 
 // --------------------------------------------------------------------------------------
+// Full-track stitch at any hop (oracle/stitch.py stitch_segments_hop), in gather form:
+//   track[src][c][t] += sum_{i in this call, covering t} w_i(t - i*hop) * seg[src][(i - i0)*C + c][t - i*hop] / E(t),
+//   E(t) = sum_{i covering t} w_i(t - i*hop) over the whole segment grid (closed form, <= ceil(L/hop) terms).
+// One thread owns one output sample: it adds this call's segments in index order and writes once -- no
+// atomics, so the result is bitwise reproducible for a given batch size at any overlap.  `seg` is the
+// model's output [S][batch*C][L] read in place (row = segment * C + channel); `track` is [S][C][n_track]
+// holding samples [track_origin, track_origin + n_track) of the full track.
+// --------------------------------------------------------------------------------------
+__device__ __forceinline__ float segment_window(long long i, int m, int seg_len, int n_seg) {
+  if ((i == 0 && m < (seg_len >> 1)) || (i == n_seg - 1 && m >= (seg_len >> 1))) return 1.f;
+  return 0.5f - 0.5f * cospif(2.0f * (float)m / (float)seg_len);
+}
+
+__global__ void __launch_bounds__(256) segment_ola_hop_kernel(const float* __restrict__ seg, int channels, int batch,
+                                                              int seg_len, int hop, int seg_index0, int n_seg_total,
+                                                              float* __restrict__ track, long long n_track,
+                                                              long long track_origin, long long j0, long long j1) {
+  const long long j = j0 + (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= j1) return;
+  const int src = blockIdx.y / channels, c = blockIdx.y - src * channels;
+  const long long t = track_origin + j;
+  const long long first = t >= seg_len ? (t - seg_len) / hop + 1 : 0;        // segments covering t: first .. last
+  const long long last = min(t / hop, (long long)n_seg_total - 1);
+  const float* in = seg + (size_t)src * batch * channels * seg_len;
+  float e = 0.f, acc = 0.f;
+  for (long long i = first; i <= last; ++i) {
+    const int m = (int)(t - i * hop);
+    const float w = segment_window(i, m, seg_len, n_seg_total);
+    e += w;
+    const long long k = i - seg_index0;
+    if (k >= 0 && k < batch) acc += w * in[((size_t)k * channels + c) * seg_len + m];
+  }
+  float* out = track + ((size_t)src * channels + c) * n_track + j;
+  *out += acc / e;
+}
+
+// --------------------------------------------------------------------------------------
 // Pair statistics for the evaluation metrics (evaluation/metrics.py:14-168): per row r of two
 // [rows, n] signals, out[r] = {sum e, sum t, sum e*e, sum t*t, sum e*t} in double.  Every metric of
 // that file (SI-SDR, SDR, "SAR", "SIR") is a closed form of these five sums, so a track never has

@@ -868,6 +868,26 @@ int tfl_segment_ola(const float* seg_audio, int n_src, int B, int seg_len, int s
   return 0;
 }
 
+int tfl_segment_ola_hop(const float* seg_audio, int rows, int channels, int B, int seg_len, int hop, int seg_index0,
+                        int n_seg_total, float* track, int64_t n_track, int64_t track_origin, tfl_stream_t stream) {
+  TFL_CHECK(seg_audio && track, "null argument");
+  TFL_CHECK(rows >= 1 && channels >= 1 && rows * (int64_t)channels <= 65535 && B >= 1 && seg_len >= 2,
+            "bad segment shape");
+  TFL_CHECK(hop >= 1 && hop < seg_len, "hop must be in [1, seg_len) (got %d for seg_len %d)", hop, seg_len);
+  TFL_CHECK(seg_index0 >= 0 && seg_index0 + B <= n_seg_total, "segment index out of range");
+  TFL_CHECK(n_track >= 0 && track_origin >= 0, "bad track range");
+  // Output samples this call touches: the span of its segments, clipped to the local buffer.
+  const int64_t lo = (int64_t)seg_index0 * hop - track_origin;
+  const int64_t hi = (int64_t)(seg_index0 + B - 1) * hop + seg_len - track_origin;
+  const int64_t j0 = lo > 0 ? lo : 0, j1 = hi < n_track ? hi : n_track;
+  if (j1 <= j0) return 0;
+  dim3 grid((unsigned)((j1 - j0 + 255) / 256), rows * channels);
+  segment_ola_hop_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(seg_audio, channels, B, seg_len, hop, seg_index0,
+                                                                 n_seg_total, track, n_track, track_origin, j0, j1);
+  TFL_LAUNCH_CHECK();
+  return 0;
+}
+
 int tfl_bs_band_split(const float* spec, int B, int M, int T, int F, int C, int nb, int max_width,
                       const int64_t* table, const float* weights, float* x, tfl_stream_t stream) {
   TFL_CHECK(spec && table && weights && x, "null argument");

@@ -266,6 +266,26 @@ def segment_ola(seg_audio: torch.Tensor, seg_index0: int, n_seg_total: int, trac
     return track
 
 
+def segment_ola_hop(seg_audio: torch.Tensor, channels: int, hop: int, seg_index0: int, n_seg_total: int,
+                    track: torch.Tensor, track_origin: int = 0):
+    """track[S, C, n] += window * seg_audio[S, B * C, seg_len] / E for segments seg_index0.. starting every ``hop``
+    samples (tfl_segment_ola_hop); row b * C + c of ``seg_audio`` is channel c of segment seg_index0 + b, and
+    ``track`` holds the samples [track_origin, track_origin + n) of the full track.  No atomics: bitwise
+    reproducible for a given batch."""
+    _require_cuda(seg_audio, "seg_audio")
+    _require_cuda(track, "track")
+    S, rows, L = seg_audio.shape
+    if (rows % channels or track.shape[:2] != (S, channels) or not track.is_contiguous()
+            or seg_audio.dtype != torch.float32 or track.dtype != torch.float32):
+        raise ValueError(f"seg_audio {tuple(seg_audio.shape)} / track {tuple(track.shape)} do not match {channels} channels")
+    lib = _lib.load()
+    with torch.cuda.device(track.device):
+        check(lib.tfl_segment_ola_hop(seg_audio.contiguous().data_ptr(), S, channels, rows // channels, L, hop,
+                                      seg_index0, n_seg_total, track.data_ptr(), track.shape[-1], track_origin,
+                                      _stream()))
+    return track
+
+
 def tc_selftest(A: torch.Tensor, B: torch.Tensor, taps: int, mode: int) -> torch.Tensor:
     """Diagnostic for the tcgen05 plumbing (tfl_tc_selftest).  mode 0: A [128+taps-1, Kd], B [taps, N, Kd];
     mode 1: A [128, Kd], B [Kd, N]; mode 3: as mode 0 in tcgen05 kind::tf32.  Returns D [128, N] fp32."""

@@ -3,16 +3,22 @@
 
     python -m mss_tf_locoformer_b200.separate --input song.wav --checkpoint model.pt [--config cfg.yaml]
         [--output_dir ./separated] [--device cuda] [--sample_rate 44100] [--seed 42]
-        [--segment 6.0] [--batch 8] [--precision bf16|fp32|tf32]
+        [--segment 6.0] [--batch 8] [--precision bf16|fp32|tf32] [--overlap 0.5] [--stereo]
 
 Same flags, same checkpoint / YAML handling, same mono down-mix, same stereo duplication and peak normalisation
 of the outputs as /root/reference/inference/separate.py:28-193 (`load_model` :79-116, `separate_audio` :119-169) and
-utils/audio.py:14-66.  Two things differ on purpose:
+utils/audio.py:14-66, by default.  Things that differ on purpose:
 
 * `--segment S` (default 6 s) runs the track as overlapping S-second segments cross-faded at 50 % overlap
   (segments.separate_track) instead of the reference's single whole-track forward, which needs memory quadratic in the
   track length (MEMORY_ANALYSIS.md:7-11).  `--segment 0` restores the reference behaviour (one forward over the track).
   Under `torchrun --nproc-per-node N` the segments are sharded over the N GPUs and rank 0 writes the files.
+* `--overlap F` (default 0.5, in (0, 1)): consecutive segments overlap by the fraction F of the segment (hop =
+  max(1, round(L * (1 - F)))).  The number of forwards grows as 1 / (1 - F): 0.75 runs twice as many as 0.5.
+* `--stereo` separates every channel of the input on its own (the model is mono) and writes [C, T] stems, peak-normalised
+  over all channels of a stem so the balance between them is kept.  Without it the input is down-mixed to mono and each
+  stem duplicated to two channels, as the reference does; a mono input gives the same output either way.
+  `--segment 0` ignores `--overlap` and `--stereo`: one forward over the down-mixed track, as the reference.
 * audio I/O uses scipy.io.wavfile (WAV only): torchaudio's codecs are not installed in this image.  Resampling uses
   scipy.signal.resample_poly, not torchaudio's windowed-sinc kernel.
 """
@@ -41,7 +47,16 @@ def parse_args(argv=None):
     p.add_argument("--segment", type=float, default=6.0, help="Segment length in seconds (0 = whole track in one forward)")
     p.add_argument("--batch", type=int, default=8, help="Segments per forward")
     p.add_argument("--precision", type=str, default="bf16", choices=["bf16", "fp32", "tf32"])
+    p.add_argument("--overlap", type=_overlap, default=0.5, help="Fraction of a segment shared with the next, in (0, 1)")
+    p.add_argument("--stereo", action="store_true", help="Separate every input channel and write multichannel stems")
     return p.parse_args(argv)
+
+
+def _overlap(text: str) -> float:
+    value = float(text)
+    if not 0.0 < value < 1.0:
+        raise argparse.ArgumentTypeError(f"overlap must be in (0, 1) (got {text})")
+    return value
 
 
 # ---- utils/audio.py:14-66 ------------------------------------------------------------------------------------------
@@ -114,19 +129,24 @@ def to_stereo(source_audio: torch.Tensor) -> torch.Tensor:
 
 
 def separate_audio(model, audio_path: str, output_dir: str, device: str = "cuda", sample_rate: int = 44100,
-                   segment: float = 6.0, batch: int = 8, rank: int = 0) -> Dict[str, str]:
-    """inference/separate.py:119-169 with segment-wise inference; returns {source: written path} (rank 0 writes)."""
+                   segment: float = 6.0, batch: int = 8, rank: int = 0, overlap: float = 0.5,
+                   stereo: bool = False) -> Dict[str, str]:
+    """inference/separate.py:119-169 with segment-wise inference; returns {source: written path} (rank 0 writes).
+    ``stereo``: separate each channel of a multichannel input and write [C, T] stems (``segment`` > 0 only)."""
     print(f"\nProcessing: {audio_path}")
     audio, sr = load_audio(audio_path, sample_rate=sample_rate, mono=False)
     print(f"Loaded audio: {audio.shape}, sample rate: {sr}")
-    mono = downmix(audio).to(device)
+    channels = stereo and segment > 0 and audio.shape[0] > 1
+    track = audio.to(device) if channels else downmix(audio).to(device)     # [C, T] or [T]
     print("Separating sources...")
     with torch.no_grad():
         seg_len = int(round(segment * sample_rate)) // 2 * 2
-        if segment > 0 and mono.shape[-1] > seg_len:
-            separated = separate_track(model, mono, seg_len=seg_len, batch=batch)
+        if segment > 0 and track.shape[-1] > seg_len:
+            separated = separate_track(model, track, seg_len=seg_len, batch=batch, overlap=overlap)
+        elif channels:
+            separated = model(track, return_time_domain=True)
         else:
-            separated = {k: v[0] for k, v in model(mono[None], return_time_domain=True).items()}
+            separated = {k: v[0] for k, v in model(track[None], return_time_domain=True).items()}
     written = {}
     if rank == 0:
         os.makedirs(output_dir, exist_ok=True)
@@ -157,7 +177,7 @@ def main(argv=None):
         model = load_model(args.checkpoint, config_path=args.config, device=device)
         model.precision = args.precision
         separate_audio(model, args.input, args.output_dir, device=device, sample_rate=args.sample_rate,
-                       segment=args.segment, batch=args.batch, rank=rank)
+                       segment=args.segment, batch=args.batch, rank=rank, overlap=args.overlap, stereo=args.stereo)
     finally:
         if world > 1:
             import torch.distributed as dist
